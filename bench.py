@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- headline benchmark of the B200 voxel frame path.
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference]
+    python bench.py --gpus N --steps K --warmup W [--impl reference] [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[2], the configuration the metric is quoted on): one full 1280x720 frame at view
 distance 12 -- chunk cull (filter A) + AABB reject / draw order (filter B) + project / near-clip / backface cull of every
@@ -164,7 +164,7 @@ def cpu_frame_baseline(sc, min_seconds: float, threads: int, steps=None, warmup=
         one_frame()
     n, t0 = 0, time.perf_counter()
     while True:
-        one_frame()
+        color, depth, _ = one_frame()
         n += 1
         el = time.perf_counter() - t0
         if steps is not None:
@@ -172,7 +172,7 @@ def cpu_frame_baseline(sc, min_seconds: float, threads: int, steps=None, warmup=
                 break
         elif el >= min_seconds:
             break
-    return n / el, n, el, int(ref.quads.size // 3)
+    return n / el, n, el, int(ref.quads.size // 3), (color, depth)
 
 
 def cpu_mesh_baseline(v, nb, min_seconds: float):
@@ -187,6 +187,23 @@ def cpu_mesh_baseline(v, nb, min_seconds: float):
     return n / el, n, el
 
 
+def dump_outputs(out_dir: str, color, depth):
+    """--dump-outputs: the frame of the last timed step, as the caller of the path receives it, in float32 (exact):
+    color_argb.npy (H, W, 4) channels A, R, G, B in 0..255 of the ARGB pixels; covered.npy (H, W) 1 where a fragment was
+    drawn, else 0; depth.npy (H, W) the depth of drawn pixels, 0 elsewhere (the frame clears depth to +inf, and every
+    stored value is finite so that outputs compare with a plain tolerance)."""
+    os.makedirs(out_dir, exist_ok=True)
+    argb = (np.asarray(color, dtype=np.uint32)[..., None] >> np.array([24, 16, 8, 0], dtype=np.uint32)) & 0xFF
+    np.save(os.path.join(out_dir, "color_argb.npy"), argb.astype(np.float32))
+    depth = np.asarray(depth, dtype=np.float32)
+    covered = np.isfinite(depth)
+    if not np.all(np.isposinf(depth[~covered])):
+        raise RuntimeError("--dump-outputs: the frame's depth holds NaN or -inf")
+    np.save(os.path.join(out_dir, "covered.npy"), covered.astype(np.float32))
+    np.save(os.path.join(out_dir, "depth.npy"), np.where(covered, depth, np.float32(0.0)))
+    log(f"outputs of the last timed step written to {out_dir}")
+
+
 def cargo_note():
     import shutil
     return "cargo found on this box but the crate's dependencies are not vendored (no network)" if shutil.which("cargo") else \
@@ -199,7 +216,9 @@ def run_reference(args):
         return 0
     sc = build_scene()
     threads = os.cpu_count() or 1
-    fps, n, el, tq = cpu_frame_baseline(sc, 0.0, threads, steps=max(1, args.steps), warmup=max(1, args.warmup))
+    fps, n, el, tq, last_frame = cpu_frame_baseline(sc, 0.0, threads, steps=max(1, args.steps), warmup=max(1, args.warmup))
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, *last_frame)
     out = {
         "impl": "reference", "metric": METRIC, "value": fps, "unit": UNIT, "n_gpus": args.gpus, "steps": n, "warmup": args.warmup,
         "ms_per_step": 1000.0 * el / n, "higher_is_better": True, "scaling": "strong", "vs_baseline": None, "dtype": "f32",
@@ -409,6 +428,13 @@ def run_cuda(args):
         extra["host_submit_us_per_frame_max_over_ranks"] = max_over_ranks(host_submit[0] / max(1, host_submit[1]) * 1e6)
     for cp in comps or []:
         cp.check()
+    last_frame = None
+    if args.dump_outputs:
+        # the last timed frame, read back from the lane that rendered it (timed_groups has synchronised the device)
+        dc, dd, rows_, width_ = api.framebuffer_device(lanes[(K - 1) % L])
+        assert (rows_, width_) == (H, W)
+        last_frame = (multigpu.device_bytes_as_tensor(dc, W * H * 4, dev).cpu().numpy().view(np.uint32).reshape(H, W),
+                      multigpu.device_bytes_as_tensor(dd, W * H * 4, dev).cpu().numpy().view(np.float32).reshape(H, W))
     # keep the same load running until the sampler has seen >= 1.5 s of it (the timed frames are ~tens of microseconds)
     t_probe = time.perf_counter()
     while time.perf_counter() - t_probe < 1.5:
@@ -875,7 +901,7 @@ def run_cuda(args):
 
     # ---- CPU baseline beside it (bounded sample) -------------------------------------------------------------------
     threads = os.cpu_count() or 1
-    cpu_fps, cpu_n, cpu_el, _ = cpu_frame_baseline(sc, 10.0, threads)
+    cpu_fps, cpu_n, cpu_el, _, _ = cpu_frame_baseline(sc, 10.0, threads)
     cpu_cps, cpu_mn, cpu_mel = cpu_mesh_baseline(v, nb, 3.0)
 
     traffic = ncu_traffic(knames[top]) if world_size == 1 else None  # the committed capture is the 1-GPU full frame
@@ -922,6 +948,8 @@ def run_cuda(args):
                                    f"(oracle/), stripe-parallel over all {threads} host threads; " + cargo_note()},
         "extra": extra,
     }
+    if last_frame is not None:
+        dump_outputs(args.dump_outputs, *last_frame)
     emit_json_line(out)
     if world_size == 1:
         del loop
@@ -1174,7 +1202,11 @@ def main():
     ap.add_argument("--composite-buffers", type=int, default=2, help="N > 1: composed-frame buffers per lane")
     ap.add_argument("--composite-depth", type=int, default=0, help="N > 1: 1 = the timed stripes also store their depth plane into GPU0's frame")
     ap.add_argument("--e2e-depth", type=int, default=0, help="frames in flight on the host in the e2e loop (default lanes, at most 2 * lanes)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the frame of the last timed step (colour channels and depth, float32 .npy) into DIR")
     args = ap.parse_args()
+    if args.dump_outputs and int(os.environ.get("WORLD_SIZE", "1")) > 1:
+        ap.error("--dump-outputs needs a one-GPU run: at N > 1 the frame is composed across ranks")
     if args.impl == "reference":
         return run_reference(args)
     return run_cuda(args)
