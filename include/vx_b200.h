@@ -421,7 +421,10 @@ VX_API int vx_render_frame_stripe(VxContext *ctx, const VxMeshBatch *batch, cons
 VX_API int vx_framebuffer_device(VxContext *ctx, uint32_t **d_color, float **d_depth, int32_t *rows, int32_t *width);
 VX_API int vx_frame_stats(VxContext *ctx, VxFrameStats *out);
 /* Diagnostics: the raw 32-word control block of the last frame -- [0] survivors, [1] quads, [2] triangles kept, [3] bin
- * entries, [4] overflow bits, [5] fullest bin, [6] big triangles (bounding box over more than 64 tiles), [7] setup units,
+ * entries, [4] overflow bits (1 triangle slots, 2 a tile bin, 8 more than 2^21 quads, 16 big-triangle list, 32 raster
+ * work items, 64 bounds check of a VX_DEBUG_CHECKS build, 128 stripe hand-off timeout, 256 setup units; a synchronous frame
+ * grows the scratch behind 1, 2, 32 and 256 and renders again, so its own word reads 0 unless the frame failed), [5] fullest
+ * bin, [6] big triangles (bounding box over more than 64 tiles), [7] setup units,
  * [8] meshes culled by the occlusion pass, [9] raster work items, [12] items the plan wanted, [13] second near-clip
  * pieces, [14] (triangle, row, column block) tasks binned, [16..24] items per plan class, [25] raster CTAs that
  * finished. */

@@ -75,3 +75,27 @@ def slice_of_quad(slice_offsets, face, k):
     so = slice_offsets[face]
     q = int(so[0]) + k
     return int(np.searchsorted(so[:33], q, side="right") - 1)
+
+
+# ---- scenes that outgrow the frame scratch a context starts with (tests/test_frame_capacity_gpu.py) ---------------------
+def chunk_plate(t=STONE, y=0):
+    """One full 32 x 32 layer of block type t: six greedy quads, the top one a single 32 x 32 face."""
+    c = empty_chunk()
+    c[:, y, :] = t
+    return c.reshape(-1)
+
+
+def chunk_checker3d_typed(t=STONE):
+    """chunk_checker3d with block type t: 98304 quads of one voxel face each."""
+    z, y, x = np.meshgrid(np.arange(32), np.arange(32), np.arange(32), indexing="ij")
+    return np.where((x + y + z) % 2 == 0, t, AIR).astype(np.uint8).reshape(-1)
+
+
+def chunk_z_plates(n=16):
+    """n layers at z = 0, 2, 4, ..., each a full 32 x 32 layer whose block type cycles with x + y + layer: no two
+    neighbouring voxels of a layer share a type, so every voxel face of a layer is a quad of its own (1024 per side)."""
+    c = empty_chunk()
+    y, x = np.meshgrid(np.arange(32), np.arange(32), indexing="ij")
+    for k in range(n):
+        c[2 * k] = (1 + (x + y + k) % 3).astype(np.uint8)
+    return c.reshape(-1)
