@@ -41,6 +41,7 @@ class Context:
         self.handle = h
         self.device = int(device)
         self._host_allocs = []
+        self._atlas = bytes(_default_atlas_cached())  # the atlas the context holds (vx_context_create loads the default one)
 
     def check(self, rc: int):
         if rc != 0:
@@ -60,6 +61,11 @@ class Context:
 
     def set_atlas(self, atlas: VxAtlas):
         self.check(self.lib.vx_set_atlas(self.handle, C.byref(atlas)))
+        self._atlas = bytes(atlas)
+
+    def holds_atlas(self, atlas: VxAtlas) -> bool:
+        """True if the last atlas loaded through set_atlas (or the default one of a new context) equals `atlas`."""
+        return self._atlas == bytes(atlas)
 
     def host_array(self, shape, dtype) -> np.ndarray:
         """Array in device-mapped page-locked host memory (vx_host_alloc): passed as color_out / depth_out of
@@ -152,6 +158,16 @@ def default_atlas() -> VxAtlas:
     a = VxAtlas()
     _lib.load().vx_default_atlas(C.byref(a))
     return a
+
+
+_default_atlas: Optional[VxAtlas] = None
+
+
+def _default_atlas_cached() -> VxAtlas:
+    global _default_atlas
+    if _default_atlas is None:
+        _default_atlas = default_atlas()
+    return _default_atlas
 
 
 def unpack_quads(q3: np.ndarray) -> np.ndarray:
@@ -471,22 +487,45 @@ class SpanWalkerRasterizer:
                                                        _p(framebuffer.depth_buffer)))
 
 
+class ShadingConfig:
+    """ShadingConfig (shading.rs:21-31): face lighting = clamp(ambient + diffuse * max(normal . light_dir, 0), 0, 1).
+    The defaults are ShadingConfig::default, the same values vx_default_frame_config writes."""
+
+    def __init__(self, light_dir=None, ambient: Optional[float] = None, diffuse: Optional[float] = None):
+        d = default_frame_config(1, 1)
+        self.light_dir = tuple(float(x) for x in (d.light_dir if light_dir is None else light_dir))
+        self.ambient = float(d.ambient if ambient is None else ambient)
+        self.diffuse = float(d.diffuse if diffuse is None else diffuse)
+
+    def apply(self, cfg: VxFrameConfig) -> VxFrameConfig:
+        cfg.light_dir[0], cfg.light_dir[1], cfg.light_dir[2] = self.light_dir
+        cfg.ambient, cfg.diffuse = self.ambient, self.diffuse
+        return cfg
+
+
 class Rasterizer:
-    """rasterizer.rs:335-431.  pub fields: backface_culling, enable_shading, shading (via frame config), atlas."""
+    """rasterizer.rs:335-431.  pub fields: backface_culling, shading, enable_shading, atlas.
+
+    Each Rasterizer draws with its own atlas (None: the default atlas, as Rasterizer::new); several of them may share a
+    context.  The context holds one atlas at a time, so a draw loads this Rasterizer's atlas first when the context
+    holds another one (vx_set_atlas; the next frame then rebuilds the colour table)."""
 
     def __init__(self, ctx: Optional[Context] = None, atlas: Optional[VxAtlas] = None):
         self.ctx = ctx or default_context()
         self.backface_culling = True
+        self.shading = ShadingConfig()
         self.enable_shading = True
+        self.atlas = atlas  # new_with_atlas rasterizer.rs:357
         self.differential_projection = False
-        if atlas is not None:  # new_with_atlas rasterizer.rs:357
-            self.ctx.set_atlas(atlas)
 
     def _cfg(self, w, h) -> VxFrameConfig:
-        cfg = default_frame_config(w, h)
+        cfg = self.shading.apply(default_frame_config(w, h))
         cfg.backface_culling = 1 if self.backface_culling else 0
         cfg.enable_shading = 1 if self.enable_shading else 0
         cfg.differential_projection = 1 if self.differential_projection else 0
+        atlas = self.atlas if self.atlas is not None else _default_atlas_cached()
+        if not self.ctx.holds_atlas(atlas):
+            self.ctx.set_atlas(atlas)
         return cfg
 
     def _render(self, batch: MeshBatch, mesh_id: int, view_proj, fb: Framebuffer, rect):

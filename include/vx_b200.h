@@ -362,7 +362,8 @@ VX_API int vx_render_frame(VxContext *ctx, const VxMeshBatch *batch, const int32
  * on a second stream, so the PCIe transfer of frame k runs beside the kernels of frame k+1 (steady-state period =
  * max(render, transfer)).  The frame's statistics and draw order are written into the slot by the frame's own kernels
  * and travel with it, so the context's next frame never waits for a transfer.  A frame whose scratch overflowed is
- * re-rendered synchronously inside _end, so the result is always the same as vx_render_frame's.
+ * re-rendered synchronously inside _end, with the cfg and the atlas (vx_set_atlas) the frame had at _begin, so the
+ * result is always the same as vx_render_frame's.
  * Frames in flight ON THE DEVICE: contexts are independent (stream + frame scratch each), so a caller that deals its
  * frames round-robin over L contexts of one device ("lanes") lets the kernels of different frames overlap -- one frame
  * is three dependent latency-bound kernels and leaves most of the GPU idle; L = 3 raises the device's frame throughput

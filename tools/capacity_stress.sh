@@ -30,7 +30,7 @@ for vd, w, h in ((12, 1280, 720), (32, 3840, 2160)):
     batch.release()
     ctx.close()
 PY
-python -m pytest tests/test_frame_gpu.py tests/test_golden.py tests/test_frame_capacity_gpu.py -m gpu -q -rA >> $LOG 2>&1
+python -m pytest tests/test_frame_gpu.py tests/test_golden.py tests/test_frame_capacity_gpu.py tests/test_atlas_shading_gpu.py -m gpu -q -rA >> $LOG 2>&1
 rc=$?
 echo "capacity-stress build ($FLAGS): rc=$rc $(tail -1 $LOG)"
 grep -E "^[0-9]+x[0-9]+ vd" $LOG

@@ -7,6 +7,6 @@ OUT=${VX_LOG_DIR:-logs}
 mkdir -p "$OUT"
 LOG=$OUT/debug_checks_${TAG}.log
 bash tools/build_variant.sh dbg "-DVX_DEBUG_CHECKS" > /dev/null 2>&1 || true
-VX_B200_LIB=$PWD/variants/libvx_dbg.so python -m pytest tests/test_frame_gpu.py tests/test_golden.py tests/test_frame_capacity_gpu.py tests/test_world_gpu.py tests/test_multi_gpu.py -m gpu -x -q > $LOG 2>&1
+VX_B200_LIB=$PWD/variants/libvx_dbg.so python -m pytest tests/test_frame_gpu.py tests/test_golden.py tests/test_frame_capacity_gpu.py tests/test_atlas_shading_gpu.py tests/test_world_gpu.py tests/test_multi_gpu.py -m gpu -x -q > $LOG 2>&1
 echo "debug-checks build: rc=$? $(tail -1 $LOG)"
 VX_B200_LIB=$PWD/variants/libvx_dbg.so python tools/sanitize_target.py >> $LOG 2>&1; echo "target rc=$?"
