@@ -117,3 +117,12 @@ inline int vx_cuda_fail(VxContext *ctx, cudaError_t e, const char *what, const c
 
 // frame scratch lifetime hooks implemented in vx_frame.cu
 void vx_frame_scratch_destroy(VxContext *ctx);
+
+// vx_multi.cu: copy a table of n <= 32 device flag pointers to ctx->multi_ptrs (again only when it differs from the last one)
+int vx_stage_flag_table(VxContext *ctx, uint32_t *const *flags, int n);
+
+// cross-GPU waits give up after timeout_us (<= 0: VX_HANDOFF_TIMEOUT_US) so that a lost peer cannot hang the device
+constexpr int32_t VX_HANDOFF_TIMEOUT_US = 2000000;
+inline unsigned long long vx_timeout_ns(int32_t timeout_us) {
+    return (unsigned long long)(timeout_us > 0 ? timeout_us : VX_HANDOFF_TIMEOUT_US) * 1000ull;
+}

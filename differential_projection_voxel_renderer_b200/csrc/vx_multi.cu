@@ -90,6 +90,17 @@ __global__ void wait_then_signal_kernel(const uint32_t *flags, int n, int stride
 
 } // namespace
 
+int vx_stage_flag_table(VxContext *ctx, uint32_t *const *flags, int n) {
+    VX_CUDA(ctx, ctx->multi_ptrs.reserve(sizeof(uint32_t *) * 32));
+    if (n > 0 && (ctx->multi_ptrs_n != n || memcmp(ctx->multi_ptrs_host, flags, sizeof(uint32_t *) * (size_t)n) != 0)) {
+        VX_CUDA(ctx, cudaStreamSynchronize(ctx->stream)); // an earlier kernel may still read the table
+        memcpy(ctx->multi_ptrs_host, flags, sizeof(uint32_t *) * (size_t)n);
+        ctx->multi_ptrs_n = n;
+        VX_CUDA(ctx, cudaMemcpyAsync(ctx->multi_ptrs.ptr, ctx->multi_ptrs_host, sizeof(uint32_t *) * (size_t)n, cudaMemcpyHostToDevice, ctx->stream));
+    }
+    return VX_OK;
+}
+
 extern "C" {
 
 int vx_device_alloc(VxContext *ctx, size_t bytes, void **d_out) {
@@ -145,14 +156,8 @@ int vx_signal_flags(VxContext *ctx, uint32_t *const *d_flags, int32_t n, uint32_
         VX_CHECK_LAUNCH(ctx);
         return VX_OK;
     }
-    // the pointer table is staged once per distinct table (tiny): keep a device copy in tmp_a
-    VX_CUDA(ctx, ctx->multi_ptrs.reserve(sizeof(uint32_t *) * 32));
-    if (memcmp(ctx->multi_ptrs_host, d_flags, sizeof(uint32_t *) * (size_t)n) != 0 || ctx->multi_ptrs_n != n) {
-        VX_CUDA(ctx, cudaStreamSynchronize(ctx->stream)); // an earlier signal may still read the table
-        memcpy(ctx->multi_ptrs_host, d_flags, sizeof(uint32_t *) * (size_t)n);
-        ctx->multi_ptrs_n = n;
-        VX_CUDA(ctx, cudaMemcpyAsync(ctx->multi_ptrs.ptr, ctx->multi_ptrs_host, sizeof(uint32_t *) * (size_t)n, cudaMemcpyHostToDevice, ctx->stream));
-    }
+    const int rc = vx_stage_flag_table(ctx, d_flags, n);
+    if (rc != VX_OK) return rc;
     signal_flags_kernel<<<1, 32, 0, ctx->stream>>>(ctx->multi_ptrs.as<uint32_t *>(), n, value);
     VX_CHECK_LAUNCH(ctx);
     return VX_OK;
@@ -166,8 +171,7 @@ int vx_wait_flags(VxContext *ctx, const uint32_t *d_flags, int32_t n, int32_t st
         VX_CUDA(ctx, ctx->multi_status.reserve(16));
         VX_CUDA(ctx, cudaMemsetAsync(ctx->multi_status.ptr, 0, 16, ctx->stream));
     }
-    const unsigned long long ns = (unsigned long long)(timeout_us > 0 ? timeout_us : 2000000) * 1000ull;
-    wait_flags_kernel<<<1, 32, 0, ctx->stream>>>(d_flags, n, stride_words, value, ns, ctx->multi_status.as<uint32_t>());
+    wait_flags_kernel<<<1, 32, 0, ctx->stream>>>(d_flags, n, stride_words, value, vx_timeout_ns(timeout_us), ctx->multi_status.as<uint32_t>());
     VX_CHECK_LAUNCH(ctx);
     return VX_OK;
 }
@@ -181,15 +185,9 @@ int vx_wait_then_signal(VxContext *ctx, const uint32_t *d_wait_flags, int32_t n_
         VX_CUDA(ctx, ctx->multi_status.reserve(16));
         VX_CUDA(ctx, cudaMemsetAsync(ctx->multi_status.ptr, 0, 16, ctx->stream));
     }
-    VX_CUDA(ctx, ctx->multi_ptrs.reserve(sizeof(uint32_t *) * 32));
-    if (n_signal > 0 && (ctx->multi_ptrs_n != n_signal || memcmp(ctx->multi_ptrs_host, d_signal_flags, sizeof(uint32_t *) * (size_t)n_signal) != 0)) {
-        VX_CUDA(ctx, cudaStreamSynchronize(ctx->stream)); // an earlier kernel may still read the table
-        memcpy(ctx->multi_ptrs_host, d_signal_flags, sizeof(uint32_t *) * (size_t)n_signal);
-        ctx->multi_ptrs_n = n_signal;
-        VX_CUDA(ctx, cudaMemcpyAsync(ctx->multi_ptrs.ptr, ctx->multi_ptrs_host, sizeof(uint32_t *) * (size_t)n_signal, cudaMemcpyHostToDevice, ctx->stream));
-    }
-    const unsigned long long ns = (unsigned long long)(timeout_us > 0 ? timeout_us : 2000000) * 1000ull;
-    wait_then_signal_kernel<<<1, 32, 0, ctx->stream>>>(d_wait_flags, n_wait, stride_words, wait_value, ns, ctx->multi_status.as<uint32_t>(),
+    const int rc = vx_stage_flag_table(ctx, d_signal_flags, n_signal);
+    if (rc != VX_OK) return rc;
+    wait_then_signal_kernel<<<1, 32, 0, ctx->stream>>>(d_wait_flags, n_wait, stride_words, wait_value, vx_timeout_ns(timeout_us), ctx->multi_status.as<uint32_t>(),
                                                        ctx->multi_ptrs.as<uint32_t *>(), n_signal, signal_value);
     VX_CHECK_LAUNCH(ctx);
     return VX_OK;
