@@ -58,14 +58,15 @@ struct VxPinnedBuffer {
 struct VxMeshBatch {
     int32_t n_chunks = 0;
     int64_t cap_quads = 0;   // capacity of d_quads in quads
-    int64_t total_quads = -1; // -1 until read back
-    int32_t n_meshes = -1;
+    // read back from the cursor on demand (vx_mesh_batch_info, which takes a const batch)
+    mutable int64_t total_quads = -1; // -1 until read back
+    mutable int32_t n_meshes = -1;
     VxDeviceBuffer quads, quad_base, quad_count, slice_offsets, face_aabb, has_mesh, positions;
-    VxDeviceBuffer cursor; // 4 x unsigned long long: quad cursor, mesh counter, overflow flag, spare
-    // world copy owned by the batch (host-array entry points only): lets vx_mesh_batch_update re-mesh edited chunks
-    // and their neighbours without re-uploading the world
+    VxDeviceBuffer cursor; // MeshCursor (vx_mesh.cu): quad cursor, mesh counter, overflow flag, work counter
+    // world copy owned by the batch (vx_mesh_chunks, vx_world_batch_create): lets vx_mesh_batch_update and
+    // vx_world_batch_remesh re-mesh chunks and their neighbours without re-uploading the world
     VxDeviceBuffer world_voxels, world_neighbors, world_flags, update_ids;
-    bool owns_world = false, has_neighbors = false, has_flags = false;
+    bool owns_world = false, has_neighbors = false;
     std::vector<int32_t> host_neighbors; // [n][6] host copy for the neighbour invalidation list
 };
 

@@ -22,6 +22,8 @@
 //            Chunks with more quads than the pool holds re-run the merge and write directly.
 #include "vx_common.cuh"
 
+#include <cstddef>
+#include <memory>
 #include <vector>
 
 namespace {
@@ -35,6 +37,14 @@ constexpr int PS = 33; // padded row stride of the 32x32 word planes (bank-confl
 constexpr int STAGE_CAP = 128;          // quads one (face, slice) unit may stage per warp on the fast path
 constexpr int POOL_CAP = 2 * 32 * PS;   // quads of a chunk kept in shared memory on the fast path (aliases P0/P1)
 constexpr unsigned FULL = 0xffffffffu;
+constexpr int SLICE_ROW = 6 * 33; // slice_offsets per chunk: 32 slice starts + the end, for each face
+constexpr int AABB_ROW = 36;      // face_aabb per chunk: min.xyz, max.xyz for each face
+
+// VxMeshBatch::cursor.  The mesh kernel takes quads from `quads`, counts non-empty meshes in `meshes`, sets `overflow` when
+// the quad stream is too small and hands out chunks beyond the first wave from `work`.
+struct MeshCursor {
+    unsigned long long quads, meshes, overflow, work;
+};
 
 struct MeshSmem {
     // stage 1: [y*PS + z], bit x = block-type bit 0 / 1.  After stage 2 the space is the chunk's quad pool.
@@ -154,7 +164,7 @@ struct ChunkArgs {
     uint32_t *quad_base, *quad_count, *slice_offsets;
     int32_t *face_aabb;
     uint8_t *has_mesh;
-    unsigned long long *cursor; // [0] quad cursor, [1] mesh counter, [2] overflow flag, [3] work counter (chunks handed out beyond the first wave)
+    MeshCursor *cursor;
 };
 
 // Neighbour solid planes.  First in load order: f=0/1 (+X/-X): i = y, bit z;  f=2/3 (+Y/-Y): i = z, bit x;
@@ -325,15 +335,15 @@ __global__ void __launch_bounds__(MESH_THREADS, VX_MESH_MIN_BLOCKS) mesh_chunks_
     int oi = blockIdx.x;
     while (oi < a.n_out) {
         __syncthreads(); // everybody is done with the previous chunk and has read next_oi
-        if (tid == 0) sm.next_oi = (int32_t)gridDim.x + (int32_t)atomicAdd(a.cursor + 3, 1ull);
+        if (tid == 0) sm.next_oi = (int32_t)gridDim.x + (int32_t)atomicAdd(&a.cursor->work, 1ull);
         do {
         const int chunk = a.subset ? a.subset[oi] : oi; // input chunk
         const int oo = a.out_by_chunk ? chunk : oi;     // where its outputs go
-        uint32_t *so = a.slice_offsets + (size_t)oo * 198;
-        int32_t *ab = a.face_aabb + (size_t)oo * 36;
+        uint32_t *so = a.slice_offsets + (size_t)oo * SLICE_ROW;
+        int32_t *ab = a.face_aabb + (size_t)oo * AABB_ROW;
         if (a.uniform_flags && a.uniform_flags[chunk]) { // Uniform chunk -> None (binary_greedy.rs:87)
-            for (int i = tid; i < 198; i += MESH_THREADS) so[i] = 0;
-            if (tid < 36) ab[tid] = (tid % 6) < 3 ? 32 : 0;
+            for (int i = tid; i < SLICE_ROW; i += MESH_THREADS) so[i] = 0;
+            if (tid < AABB_ROW) ab[tid] = (tid % 6) < 3 ? 32 : 0;
             if (tid == 0) {
                 a.quad_base[oo] = 0;
                 a.quad_count[oo] = 0;
@@ -418,11 +428,11 @@ __global__ void __launch_bounds__(MESH_THREADS, VX_MESH_MIN_BLOCKS) mesh_chunks_
             sm.total = run;
             unsigned long long base = 0;
             if (run) {
-                base = atomicAdd(a.cursor, (unsigned long long)run);
-                atomicAdd(a.cursor + 1, 1ull);
+                base = atomicAdd(&a.cursor->quads, (unsigned long long)run);
+                atomicAdd(&a.cursor->meshes, 1ull);
             }
             sm.overflow = (base + run > a.cap_quads) ? 1u : 0u;
-            if (sm.overflow) atomicExch(a.cursor + 2, 1ull);
+            if (sm.overflow) atomicExch(&a.cursor->overflow, 1ull);
             sm.base = (uint32_t)base;
             a.quad_base[oo] = (uint32_t)base;
             a.quad_count[oo] = run;
@@ -489,36 +499,97 @@ __global__ void greedy_slices_kernel(const uint32_t *masks, int n, VxQuad *out, 
     if (lane == 0) n_out[w] = (int32_t)c;
 }
 
-int batch_alloc(VxContext *ctx, VxMeshBatch *b, int32_t n, int64_t cap_quads) {
+// The per-chunk arrays of a batch: bytes per chunk, and the byte that marks an absent chunk of a world batch.  Every batch
+// has the first MESH_ARRAYS; a batch that owns its world copy (vx_mesh_chunks, vx_world_batch_create) has all of them.
+struct ChunkArray {
+    VxDeviceBuffer VxMeshBatch::*buf;
+    size_t row_bytes;
+    int absent;
+};
+constexpr ChunkArray CHUNK_ARRAYS[] = {
+    {&VxMeshBatch::quad_base, sizeof(uint32_t), 0},
+    {&VxMeshBatch::quad_count, sizeof(uint32_t), 0},
+    {&VxMeshBatch::slice_offsets, sizeof(uint32_t) * SLICE_ROW, 0},
+    {&VxMeshBatch::face_aabb, sizeof(int32_t) * AABB_ROW, 0},
+    {&VxMeshBatch::has_mesh, 1, 0},
+    {&VxMeshBatch::positions, sizeof(int32_t) * 3, 0},
+    {&VxMeshBatch::world_voxels, VX_CHUNK_VOLUME, 0},
+    {&VxMeshBatch::world_neighbors, sizeof(int32_t) * 6, 0xFF}, // VX_NBR_NONE
+    {&VxMeshBatch::world_flags, 1, 1},                          // "uniform air"
+};
+constexpr int MESH_ARRAYS = 6, ALL_ARRAYS = sizeof(CHUNK_ARRAYS) / sizeof(CHUNK_ARRAYS[0]);
+
+struct BatchRelease {
+    VxContext *ctx;
+    void operator()(VxMeshBatch *b) const { vx_mesh_batch_release(ctx, b); }
+};
+// a batch under construction: released on every failure exit, handed to the caller with release()
+using BatchPtr = std::unique_ptr<VxMeshBatch, BatchRelease>;
+
+// quad stream of a batch that is about to be meshed: a typical terrain chunk has ~200 quads (binary_greedy.rs:91), so start
+// with 512 per chunk and regrow on demand
+int64_t first_cap_quads(int32_t n) { return (int64_t)(n > 0 ? n : 1) * 512; }
+
+// A new batch of n chunks with the first `arrays` of CHUNK_ARRAYS, the cursor and room for cap_quads quads.
+int new_batch(VxContext *ctx, int32_t n, int64_t cap_quads, int arrays, BatchPtr &b) {
+    b = BatchPtr(new VxMeshBatch(), BatchRelease{ctx});
     b->n_chunks = n;
-    VX_CUDA(ctx, b->quad_base.reserve(sizeof(uint32_t) * (size_t)n));
-    VX_CUDA(ctx, b->quad_count.reserve(sizeof(uint32_t) * (size_t)n));
-    VX_CUDA(ctx, b->slice_offsets.reserve(sizeof(uint32_t) * 198 * (size_t)n));
-    VX_CUDA(ctx, b->face_aabb.reserve(sizeof(int32_t) * 36 * (size_t)n));
-    VX_CUDA(ctx, b->has_mesh.reserve((size_t)n));
-    VX_CUDA(ctx, b->positions.reserve(sizeof(int32_t) * 3 * (size_t)n));
-    VX_CUDA(ctx, b->cursor.reserve(sizeof(unsigned long long) * 4));
+    for (int k = 0; k < arrays; ++k) VX_CUDA(ctx, (b.get()->*CHUNK_ARRAYS[k].buf).reserve(CHUNK_ARRAYS[k].row_bytes * (size_t)n));
+    VX_CUDA(ctx, b->cursor.reserve(sizeof(MeshCursor)));
     VX_CUDA(ctx, b->quads.reserve(3 * (size_t)cap_quads + 16));
     b->cap_quads = cap_quads;
     return VX_OK;
 }
 
-// append = true: in-place update of the chunks in d_subset (n_sub of them): outputs at the chunks' own indices, new
-// quads appended behind the current end of the quad stream (the old ones become dead space).
-int run_mesher(VxContext *ctx, const uint8_t *d_vox, const int32_t *d_nb, const uint8_t *d_uf, VxMeshBatch *b,
-               bool allow_regrow, const int32_t *d_subset = nullptr, int32_t n_total = -1, bool append = false,
-               int32_t n_sub = 0) {
+int read_cursor(VxContext *ctx, const VxMeshBatch *b, MeshCursor &h) {
+    VX_CUDA(ctx, cudaMemcpyAsync(&h, b->cursor.ptr, sizeof(h), cudaMemcpyDeviceToHost, ctx->stream));
+    VX_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+    return VX_OK;
+}
+
+// also waits for everything enqueued before it (h and the caller's host arrays may go out of scope)
+int write_cursor(VxContext *ctx, VxMeshBatch *b, const MeshCursor &h) {
+    VX_CUDA(ctx, cudaMemcpyAsync(b->cursor.ptr, &h, sizeof(h), cudaMemcpyHostToDevice, ctx->stream));
+    VX_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+    return VX_OK;
+}
+
+// What the mesher reads: the voxels of n_chunks chunks, their neighbour rows (null: all VX_NBR_NONE) and Uniform flags
+// (null: all Varied).  Neighbour indices refer to these n_chunks.
+struct MeshInput {
+    const uint8_t *voxels;
+    const int32_t *neighbors;
+    const uint8_t *uniform_flags;
+    int32_t n_chunks;
+};
+
+MeshInput world_input(const VxMeshBatch *b) {
+    return {b->world_voxels.as<uint8_t>(), b->has_neighbors ? b->world_neighbors.as<int32_t>() : nullptr, b->world_flags.as<uint8_t>(),
+            b->n_chunks};
+}
+
+enum class MeshMode {
+    EveryRowRegrow, // every row; the cursor is read back, and an overflowed quad stream is grown to the exact need and meshed again
+    EveryRowSteady, // every row, no read-back: an overflow is reported by the next vx_mesh_batch_info
+    AppendListed,   // the listed chunks at their own rows, quads appended behind the stream's end (their old quads become dead space)
+};
+
+// Every-row modes: row i of the batch is chunk rows[i] of `in` (chunk i when rows is null), n_rows == b->n_chunks.
+// AppendListed: rows lists the n_rows chunks to re-mesh.
+int run_mesher(VxContext *ctx, VxMeshBatch *b, const MeshInput &in, MeshMode mode, const int32_t *rows, int32_t n_rows) {
+    const bool listed = mode == MeshMode::AppendListed;
+    MeshCursor *cursor = b->cursor.as<MeshCursor>();
     for (int attempt = 0; attempt < 2; ++attempt) {
-        if (!append) VX_CUDA(ctx, cudaMemsetAsync(b->cursor.ptr, 0, sizeof(unsigned long long) * 4, ctx->stream));
-        else VX_CUDA(ctx, cudaMemsetAsync(b->cursor.as<unsigned long long>() + 3, 0, sizeof(unsigned long long), ctx->stream)); // work counter
+        if (listed) VX_CUDA(ctx, cudaMemsetAsync(&cursor->work, 0, sizeof(cursor->work), ctx->stream));
+        else VX_CUDA(ctx, cudaMemsetAsync(cursor, 0, sizeof(MeshCursor), ctx->stream));
         ChunkArgs a;
-        a.voxels = d_vox;
-        a.neighbors = d_nb;
-        a.uniform_flags = d_uf;
-        a.n_chunks = n_total >= 0 ? n_total : b->n_chunks;
-        a.subset = d_subset;
-        a.n_out = append ? n_sub : b->n_chunks;
-        a.out_by_chunk = append ? 1 : 0;
+        a.voxels = in.voxels;
+        a.neighbors = in.neighbors;
+        a.uniform_flags = in.uniform_flags;
+        a.n_chunks = in.n_chunks;
+        a.subset = rows;
+        a.n_out = n_rows;
+        a.out_by_chunk = listed ? 1 : 0;
         a.quads = b->quads.as<uint8_t>();
         a.cap_quads = (unsigned long long)b->cap_quads;
         a.quad_base = b->quad_base.as<uint32_t>();
@@ -526,7 +597,7 @@ int run_mesher(VxContext *ctx, const uint8_t *d_vox, const int32_t *d_nb, const 
         a.slice_offsets = b->slice_offsets.as<uint32_t>();
         a.face_aabb = b->face_aabb.as<int32_t>();
         a.has_mesh = b->has_mesh.as<uint8_t>();
-        a.cursor = b->cursor.as<unsigned long long>();
+        a.cursor = cursor;
         int per_sm = 0;
         VX_CUDA(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, mesh_chunks_kernel, MESH_THREADS, 0));
         if (per_sm < 1) per_sm = 1;
@@ -537,31 +608,51 @@ int run_mesher(VxContext *ctx, const uint8_t *d_vox, const int32_t *d_nb, const 
         VX_CHECK_LAUNCH(ctx);
         b->total_quads = -1;
         b->n_meshes = -1;
-        if (!allow_regrow || append) return VX_OK;
-        unsigned long long h[4];
-        VX_CUDA(ctx, cudaMemcpyAsync(h, b->cursor.ptr, sizeof(h), cudaMemcpyDeviceToHost, ctx->stream));
-        VX_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-        if (!h[2]) {
-            b->total_quads = (int64_t)h[0];
-            b->n_meshes = (int32_t)h[1];
+        if (mode != MeshMode::EveryRowRegrow) return VX_OK;
+        MeshCursor h;
+        const int rc = read_cursor(ctx, b, h);
+        if (rc != VX_OK) return rc;
+        if (!h.overflow) {
+            b->total_quads = (int64_t)h.quads;
+            b->n_meshes = (int32_t)h.meshes;
             return VX_OK;
         }
-        if (h[0] >= (1ull << 32)) return vx_fail(ctx, VX_ERR_CAPACITY, "more than 2^32 quads in one batch");
-        // quad stream was too small: grow to the exact need and re-run
-        VX_CUDA(ctx, b->quads.reserve(3 * (size_t)h[0] + 16));
-        b->cap_quads = (int64_t)h[0];
+        if (h.quads >= (1ull << 32)) return vx_fail(ctx, VX_ERR_CAPACITY, "more than 2^32 quads in one batch");
+        VX_CUDA(ctx, b->quads.reserve(3 * (size_t)h.quads + 16));
+        b->cap_quads = (int64_t)h.quads;
     }
     return vx_fail(ctx, VX_ERR_CAPACITY, "mesher output did not fit after regrow");
+}
+
+// Mesh every row of a new batch (EveryRowRegrow; an empty batch has nothing to mesh) and hand it to *out.
+int mesh_new_batch(VxContext *ctx, BatchPtr &b, const MeshInput &in, const int32_t *rows, VxMeshBatch **out) {
+    if (b->n_chunks > 0) {
+        const int rc = run_mesher(ctx, b.get(), in, MeshMode::EveryRowRegrow, rows, b->n_chunks);
+        if (rc != VX_OK) return rc;
+    } else {
+        b->total_quads = 0;
+        b->n_meshes = 0;
+    }
+    *out = b.release();
+    return VX_OK;
+}
+
+// positions of the batch's chunks from the device array d_positions, or zeros without one
+int copy_positions(VxContext *ctx, VxMeshBatch *b, const int32_t *d_positions) {
+    const size_t bytes = sizeof(int32_t) * 3 * (size_t)b->n_chunks;
+    if (bytes == 0) return VX_OK;
+    if (d_positions) VX_CUDA(ctx, cudaMemcpyAsync(b->positions.ptr, d_positions, bytes, cudaMemcpyDeviceToDevice, ctx->stream));
+    else VX_CUDA(ctx, cudaMemsetAsync(b->positions.ptr, 0, bytes, ctx->stream));
+    return VX_OK;
 }
 
 struct ShardOffsets {
     uint32_t off[64]; // first quad of rank r's stream in the assembled stream
 };
 
-// one CTA per chunk of the assembled batch: copy its row from the gathered shard blocks (vx_mesh_batch_assemble_shards)
 // first quad of every rank's stream in the assembled stream, from the totals the blocks carry (no host round trip): one thread
 __global__ void shard_offsets_kernel(int world, const uint8_t *__restrict__ blocks, VxShardLayout L, uint32_t *off /* [64] offsets, [64] totals */,
-                                     unsigned long long *cursor, unsigned long long cap_quads) {
+                                     MeshCursor *cursor, unsigned long long cap_quads) {
     if (blockIdx.x != 0 || threadIdx.x != 0) return;
     unsigned long long run = 0, overflow = 0;
     for (int r = 0; r < world; ++r) {
@@ -575,10 +666,10 @@ __global__ void shard_offsets_kernel(int world, const uint8_t *__restrict__ bloc
         run += t;
     }
     if (run > cap_quads || run >= (1ull << 32)) overflow = 1;
-    cursor[0] = run;
-    cursor[1] = 0; // meshes: counted by the assemble kernel
-    cursor[2] = overflow;
-    cursor[3] = 0;
+    cursor->quads = run;
+    cursor->meshes = 0; // counted by the assemble kernel
+    cursor->overflow = overflow;
+    cursor->work = 0;
 }
 
 // one thread per quad of every rank's stream: move it to its place in the assembled stream
@@ -595,9 +686,10 @@ __global__ void __launch_bounds__(256) copy_shard_quads_kernel(const uint8_t *__
     }
 }
 
+// one CTA per chunk of the assembled batch: copy its row from the gathered shard blocks (vx_mesh_batch_assemble_shards)
 __global__ void __launch_bounds__(64) assemble_shards_kernel(int n_chunks, int world, ShardOffsets so, const uint8_t *__restrict__ blocks, VxShardLayout L,
                                                              uint32_t *quad_base, uint32_t *quad_count, uint32_t *slice_offsets, int32_t *face_aabb,
-                                                             uint8_t *has_mesh, unsigned long long *cursor, unsigned long long total,
+                                                             uint8_t *has_mesh, MeshCursor *cursor, unsigned long long total,
                                                              const uint32_t *__restrict__ d_off = nullptr) {
     const int c = blockIdx.x;
     if (c >= n_chunks) return;
@@ -608,20 +700,56 @@ __global__ void __launch_bounds__(64) assemble_shards_kernel(int n_chunks, int w
     const uint32_t *g_so = reinterpret_cast<const uint32_t *>(blk + L.off_slice_offsets);
     const int32_t *g_aabb = reinterpret_cast<const int32_t *>(blk + L.off_face_aabb);
     const uint8_t *g_has = blk + L.off_has_mesh;
-    for (int i = threadIdx.x; i < 198; i += 64) slice_offsets[(size_t)c * 198 + i] = g_so[j * 198 + i];
-    if (threadIdx.x < 36) face_aabb[(size_t)c * 36 + threadIdx.x] = g_aabb[j * 36 + threadIdx.x];
-    if (threadIdx.x == 36) quad_base[c] = g_base[j] + (d_off ? d_off[r] : so.off[r]);
-    if (threadIdx.x == 37) quad_count[c] = g_count[j];
-    if (threadIdx.x == 38) {
+    for (int i = threadIdx.x; i < SLICE_ROW; i += 64) slice_offsets[(size_t)c * SLICE_ROW + i] = g_so[j * SLICE_ROW + i];
+    if (threadIdx.x < AABB_ROW) face_aabb[(size_t)c * AABB_ROW + threadIdx.x] = g_aabb[j * AABB_ROW + threadIdx.x];
+    if (threadIdx.x == AABB_ROW) quad_base[c] = g_base[j] + (d_off ? d_off[r] : so.off[r]);
+    if (threadIdx.x == AABB_ROW + 1) quad_count[c] = g_count[j];
+    if (threadIdx.x == AABB_ROW + 2) {
         has_mesh[c] = g_has[j];
-        if (d_off && g_has[j]) atomicAdd(cursor + 1, 1ull);
+        if (d_off && g_has[j]) atomicAdd(&cursor->meshes, 1ull);
     }
-    if (!d_off && c == 0 && threadIdx.x == 39) {
-        cursor[0] = total;
-        cursor[1] = 0;
-        cursor[2] = 0;
-        cursor[3] = 0;
+    if (!d_off && c == 0 && threadIdx.x == AABB_ROW + 3) {
+        cursor->quads = total;
+        cursor->meshes = 0;
+        cursor->overflow = 0;
+        cursor->work = 0;
     }
+}
+
+// The batch an assemble of n_chunks writes: *batch_inout (created for the same n_chunks; its quad stream grown to `want`
+// quads after a synchronise when it holds fewer than `need`), or a new one with room for `want`, owned by `fresh`.  The
+// positions are copied from d_positions; a new batch without them gets zeros.
+int assemble_target(VxContext *ctx, VxMeshBatch *const *batch_inout, int32_t n_chunks, int64_t need, int64_t want,
+                    const int32_t *d_positions, BatchPtr &fresh) {
+    VxMeshBatch *b = *batch_inout;
+    if (!b) {
+        const int rc = new_batch(ctx, n_chunks, want > 0 ? want : 1, MESH_ARRAYS, fresh);
+        if (rc != VX_OK) return rc;
+        b = fresh.get();
+    } else if (b->n_chunks != n_chunks) {
+        return vx_fail(ctx, VX_ERR_INVALID, "batch was created for another chunk count");
+    } else if (need > b->cap_quads) {
+        VX_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+        VX_CUDA(ctx, b->quads.reserve(3 * (size_t)want + 16));
+        b->cap_quads = want;
+    }
+    return d_positions || fresh ? copy_positions(ctx, b, d_positions) : VX_OK;
+}
+
+// device-to-device copy into a shard block (nothing for an empty section)
+cudaError_t to_block(VxContext *ctx, uint8_t *d_block, int64_t off, const void *src, size_t bytes) {
+    return bytes ? cudaMemcpyAsync(d_block + off, src, bytes, cudaMemcpyDeviceToDevice, ctx->stream) : cudaSuccess;
+}
+
+// the shard's per-chunk arrays into their sections of the block (vx_shard_layout)
+int pack_rows(VxContext *ctx, const VxMeshBatch *shard, const VxShardLayout *L, uint8_t *d_block) {
+    const size_t n = (size_t)shard->n_chunks;
+    VX_CUDA(ctx, to_block(ctx, d_block, L->off_quad_base, shard->quad_base.ptr, 4 * n));
+    VX_CUDA(ctx, to_block(ctx, d_block, L->off_quad_count, shard->quad_count.ptr, 4 * n));
+    VX_CUDA(ctx, to_block(ctx, d_block, L->off_slice_offsets, shard->slice_offsets.ptr, 4 * SLICE_ROW * n));
+    VX_CUDA(ctx, to_block(ctx, d_block, L->off_face_aabb, shard->face_aabb.ptr, 4 * AABB_ROW * n));
+    VX_CUDA(ctx, to_block(ctx, d_block, L->off_has_mesh, shard->has_mesh.ptr, n));
+    return VX_OK;
 }
 
 // one CTA per live chunk: move its quads from the old stream to their place in the compacted one
@@ -671,28 +799,40 @@ int compact_stream(VxContext *ctx, VxMeshBatch *b, int64_t extra_quads) {
         VX_CHECK_LAUNCH(ctx);
     }
     if (n) VX_CUDA(ctx, cudaMemcpyAsync(b->quad_base.ptr, base.data(), 4 * n, cudaMemcpyHostToDevice, ctx->stream));
-    unsigned long long h[4] = {live, 0ull, 0ull, 0ull};
-    for (size_t i = 0; i < n; ++i) h[1] += has[i] ? 1 : 0;
-    VX_CUDA(ctx, cudaMemcpyAsync(b->cursor.ptr, h, sizeof(h), cudaMemcpyHostToDevice, ctx->stream));
-    VX_CUDA(ctx, cudaStreamSynchronize(ctx->stream)); // the host vectors above go out of scope
+    MeshCursor h{live, 0ull, 0ull, 0ull};
+    for (size_t i = 0; i < n; ++i) h.meshes += has[i] ? 1 : 0;
+    const int rc = write_cursor(ctx, b, h); // also waits for the copies from the host vectors above
+    if (rc != VX_OK) return rc;
     b->quads.release();
     b->quads = fresh;
     b->cap_quads = want;
     b->total_quads = (int64_t)live;
-    b->n_meshes = (int32_t)h[1];
+    b->n_meshes = (int32_t)h.meshes;
     return VX_OK;
 }
 
-// re-mesh exactly the listed chunks of a world-owning batch in place (append + compaction when the stream is full)
+// ids (in range) without repeats, in first-seen order
+std::vector<int32_t> unique_ids(const std::vector<int32_t> &ids, int32_t n_chunks) {
+    std::vector<int32_t> list;
+    std::vector<uint8_t> seen((size_t)n_chunks, 0);
+    for (const int32_t c : ids)
+        if (!seen[c]) {
+            seen[c] = 1;
+            list.push_back(c);
+        }
+    return list;
+}
+
+// Re-mesh exactly the listed chunks of a world-owning batch in place.  Their quads are appended behind the live end of
+// the stream; when it has no room for them, the live quads are compacted first (copied, not re-meshed), so every other
+// chunk's mesh stays as it is.
 int remesh_listed(VxContext *ctx, VxMeshBatch *b, const std::vector<int32_t> &list) {
     if (list.empty()) return VX_OK;
-    const uint8_t *d_vox = b->world_voxels.as<uint8_t>();
-    const int32_t *d_nb = b->has_neighbors ? b->world_neighbors.as<int32_t>() : nullptr;
-    const uint8_t *d_uf = b->world_flags.as<uint8_t>();
     VxMeshBatchInfo info;
     int rc = vx_mesh_batch_info(ctx, b, &info);
     if (rc != VX_OK) return rc;
     for (int attempt = 0; attempt < 3; ++attempt) {
+        // typical chunk: a few hundred quads, so 4096 each is a generous bound that the overflow flag backs up
         const int64_t room = (int64_t)list.size() * (attempt == 0 ? 4096 : 98304); // 98,304 = the most quads a chunk can have
         if (b->total_quads + room > b->cap_quads) {
             rc = compact_stream(ctx, b, room);
@@ -701,21 +841,21 @@ int remesh_listed(VxContext *ctx, VxMeshBatch *b, const std::vector<int32_t> &li
         const int64_t before = b->total_quads; // live end of the stream (run_mesher invalidates the cached value)
         VX_CUDA(ctx, b->update_ids.reserve(sizeof(int32_t) * list.size()));
         VX_CUDA(ctx, cudaMemcpyAsync(b->update_ids.ptr, list.data(), sizeof(int32_t) * list.size(), cudaMemcpyHostToDevice, ctx->stream));
-        rc = run_mesher(ctx, d_vox, d_nb, d_uf, b, false, b->update_ids.as<int32_t>(), b->n_chunks, true, (int32_t)list.size());
+        rc = run_mesher(ctx, b, world_input(b), MeshMode::AppendListed, b->update_ids.as<int32_t>(), (int32_t)list.size());
         if (rc != VX_OK) return rc;
-        unsigned long long h[4];
-        VX_CUDA(ctx, cudaMemcpyAsync(h, b->cursor.ptr, sizeof(h), cudaMemcpyDeviceToHost, ctx->stream));
-        VX_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-        if (!h[2]) {
-            b->total_quads = (int64_t)h[0];
-            b->n_meshes = -1;
+        MeshCursor h;
+        rc = read_cursor(ctx, b, h);
+        if (rc != VX_OK) return rc;
+        if (!h.overflow) {
+            b->total_quads = (int64_t)h.quads; // length of the stream, dead space included
+            b->n_meshes = -1;                  // recounted on demand
             return VX_OK;
         }
         // overflow: the chunks of this list that did not fit have no quads; clear the flag, make room, mesh the list again
-        h[2] = 0;
-        h[0] = (unsigned long long)before;
-        VX_CUDA(ctx, cudaMemcpyAsync(b->cursor.ptr, h, sizeof(h), cudaMemcpyHostToDevice, ctx->stream));
-        VX_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+        h.overflow = 0;
+        h.quads = (unsigned long long)before;
+        rc = write_cursor(ctx, b, h);
+        if (rc != VX_OK) return rc;
         b->total_quads = before;
     }
     return vx_fail(ctx, VX_ERR_CAPACITY, "world batch: quad stream overflow persisted");
@@ -731,26 +871,11 @@ int vx_mesh_chunks_device(VxContext *ctx, const uint8_t *d_voxels, const int32_t
     if (!ctx || !out || n_chunks < 0 || (n_chunks > 0 && !d_voxels)) return vx_fail(ctx, VX_ERR_INVALID, "vx_mesh_chunks_device: bad argument");
     if ((reinterpret_cast<uintptr_t>(d_voxels) & 15) != 0) return vx_fail(ctx, VX_ERR_INVALID, "voxels must be 16-byte aligned");
     VX_CUDA(ctx, cudaSetDevice(ctx->device));
-    VxMeshBatch *b = new VxMeshBatch();
-    // typical terrain chunk: ~200 quads (binary_greedy.rs:91); start with 512 per chunk, regrow on demand
-    int rc = batch_alloc(ctx, b, n_chunks, (int64_t)(n_chunks > 0 ? n_chunks : 1) * 512);
-    if (rc == VX_OK && n_chunks > 0) {
-        if (d_positions) {
-            cudaError_t e = cudaMemcpyAsync(b->positions.ptr, d_positions, sizeof(int32_t) * 3 * (size_t)n_chunks,
-                                            cudaMemcpyDeviceToDevice, ctx->stream);
-            if (e != cudaSuccess) rc = vx_cuda_fail(ctx, e, "copy positions", __FILE__, __LINE__);
-        } else {
-            cudaMemsetAsync(b->positions.ptr, 0, sizeof(int32_t) * 3 * (size_t)n_chunks, ctx->stream);
-        }
-    }
-    if (rc == VX_OK && n_chunks > 0) rc = run_mesher(ctx, d_voxels, d_neighbors, d_uniform_flags, b, true);
-    if (rc == VX_OK && n_chunks == 0) { b->total_quads = 0; b->n_meshes = 0; }
-    if (rc != VX_OK) {
-        vx_mesh_batch_release(ctx, b);
-        return rc;
-    }
-    *out = b;
-    return VX_OK;
+    BatchPtr b;
+    int rc = new_batch(ctx, n_chunks, first_cap_quads(n_chunks), MESH_ARRAYS, b);
+    if (rc == VX_OK) rc = copy_positions(ctx, b.get(), d_positions);
+    if (rc == VX_OK) rc = mesh_new_batch(ctx, b, {d_voxels, d_neighbors, d_uniform_flags, n_chunks}, nullptr, out);
+    return rc;
 }
 
 int vx_mesh_chunk_subset_device(VxContext *ctx, const uint8_t *d_voxels, const int32_t *d_positions,
@@ -760,41 +885,31 @@ int vx_mesh_chunk_subset_device(VxContext *ctx, const uint8_t *d_voxels, const i
         return vx_fail(ctx, VX_ERR_INVALID, "vx_mesh_chunk_subset_device: bad argument");
     if ((reinterpret_cast<uintptr_t>(d_voxels) & 15) != 0) return vx_fail(ctx, VX_ERR_INVALID, "voxels must be 16-byte aligned");
     VX_CUDA(ctx, cudaSetDevice(ctx->device));
+    const MeshInput in{d_voxels, d_neighbors, d_uniform_flags, n_chunks};
     if (*batch_inout) { // steady state: re-mesh the same shard into the existing batch, no allocation
         if ((*batch_inout)->n_chunks != n_subset) return vx_fail(ctx, VX_ERR_INVALID, "batch was created for another subset size");
         if (n_subset == 0) return VX_OK;
-        return run_mesher(ctx, d_voxels, d_neighbors, d_uniform_flags, *batch_inout, false, d_subset, n_chunks);
+        return run_mesher(ctx, *batch_inout, in, MeshMode::EveryRowSteady, d_subset, n_subset);
     }
-    VxMeshBatch *b = new VxMeshBatch();
-    int rc = batch_alloc(ctx, b, n_subset, (int64_t)(n_subset > 0 ? n_subset : 1) * 512);
-    if (rc == VX_OK && n_subset > 0) {
-        // positions of the subset, gathered on the host side of the stream (small)
-        if (d_positions) {
-            std::vector<int32_t> ids((size_t)n_subset), pos((size_t)n_chunks * 3), sub((size_t)n_subset * 3);
-            cudaError_t e = cudaMemcpyAsync(ids.data(), d_subset, sizeof(int32_t) * (size_t)n_subset, cudaMemcpyDeviceToHost, ctx->stream);
-            if (e == cudaSuccess) e = cudaMemcpyAsync(pos.data(), d_positions, sizeof(int32_t) * 3 * (size_t)n_chunks, cudaMemcpyDeviceToHost, ctx->stream);
-            if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
-            if (e == cudaSuccess) {
-                for (int32_t i = 0; i < n_subset; ++i) {
-                    if (ids[i] < 0 || ids[i] >= n_chunks) { rc = vx_fail(ctx, VX_ERR_INVALID, "subset id out of range"); break; }
-                    for (int k = 0; k < 3; ++k) sub[(size_t)i * 3 + k] = pos[(size_t)ids[i] * 3 + k];
-                }
-                if (rc == VX_OK) e = cudaMemcpyAsync(b->positions.ptr, sub.data(), sizeof(int32_t) * 3 * (size_t)n_subset, cudaMemcpyHostToDevice, ctx->stream);
-                if (rc == VX_OK && e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
-            }
-            if (rc == VX_OK && e != cudaSuccess) rc = vx_cuda_fail(ctx, e, "subset positions", __FILE__, __LINE__);
-        } else {
-            cudaMemsetAsync(b->positions.ptr, 0, sizeof(int32_t) * 3 * (size_t)n_subset, ctx->stream);
+    BatchPtr b;
+    int rc = new_batch(ctx, n_subset, first_cap_quads(n_subset), MESH_ARRAYS, b);
+    if (rc != VX_OK) return rc;
+    if (d_positions && n_subset > 0) { // positions of the subset, gathered on the host side of the stream (small)
+        std::vector<int32_t> ids((size_t)n_subset), pos((size_t)n_chunks * 3), sub((size_t)n_subset * 3);
+        VX_CUDA(ctx, cudaMemcpyAsync(ids.data(), d_subset, sizeof(int32_t) * (size_t)n_subset, cudaMemcpyDeviceToHost, ctx->stream));
+        VX_CUDA(ctx, cudaMemcpyAsync(pos.data(), d_positions, sizeof(int32_t) * 3 * (size_t)n_chunks, cudaMemcpyDeviceToHost, ctx->stream));
+        VX_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+        for (int32_t i = 0; i < n_subset; ++i) {
+            if (ids[i] < 0 || ids[i] >= n_chunks) return vx_fail(ctx, VX_ERR_INVALID, "subset id out of range");
+            for (int k = 0; k < 3; ++k) sub[(size_t)i * 3 + k] = pos[(size_t)ids[i] * 3 + k];
         }
+        VX_CUDA(ctx, cudaMemcpyAsync(b->positions.ptr, sub.data(), sizeof(int32_t) * 3 * (size_t)n_subset, cudaMemcpyHostToDevice, ctx->stream));
+        VX_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+    } else {
+        rc = copy_positions(ctx, b.get(), nullptr);
+        if (rc != VX_OK) return rc;
     }
-    if (rc == VX_OK && n_subset > 0) rc = run_mesher(ctx, d_voxels, d_neighbors, d_uniform_flags, b, true, d_subset, n_chunks);
-    if (rc == VX_OK && n_subset == 0) { b->total_quads = 0; b->n_meshes = 0; }
-    if (rc != VX_OK) {
-        vx_mesh_batch_release(ctx, b);
-        return rc;
-    }
-    *batch_inout = b;
-    return VX_OK;
+    return mesh_new_batch(ctx, b, in, d_subset, batch_inout);
 }
 
 int vx_remesh_chunks_device(VxContext *ctx, const uint8_t *d_voxels, const int32_t *d_neighbors,
@@ -802,7 +917,7 @@ int vx_remesh_chunks_device(VxContext *ctx, const uint8_t *d_voxels, const int32
     if (!ctx || !batch || !d_voxels) return vx_fail(ctx, VX_ERR_INVALID, "vx_remesh_chunks_device: bad argument");
     if (batch->n_chunks == 0) return VX_OK;
     VX_CUDA(ctx, cudaSetDevice(ctx->device));
-    return run_mesher(ctx, d_voxels, d_neighbors, d_uniform_flags, batch, false);
+    return run_mesher(ctx, batch, {d_voxels, d_neighbors, d_uniform_flags, batch->n_chunks}, MeshMode::EveryRowSteady, nullptr, batch->n_chunks);
 }
 
 int vx_mesh_chunks(VxContext *ctx, const uint8_t *voxels, const int32_t *positions, const int32_t *neighbors,
@@ -811,31 +926,21 @@ int vx_mesh_chunks(VxContext *ctx, const uint8_t *voxels, const int32_t *positio
     VX_CUDA(ctx, cudaSetDevice(ctx->device));
     const size_t n = (size_t)n_chunks;
     // the world copy stays with the batch (vx_mesh_batch_update edits it in place)
-    VxDeviceBuffer wv, wn, wf;
-    VX_CUDA(ctx, wv.reserve(n * VX_CHUNK_VOLUME + 16));
-    VX_CUDA(ctx, wn.reserve(n * 6 * sizeof(int32_t) + 16));
-    VX_CUDA(ctx, wf.reserve(n + 16));
-    VX_CUDA(ctx, ctx->tmp_d.reserve(n * 3 * sizeof(int32_t) + 16));
-    if (n) VX_CUDA(ctx, cudaMemcpyAsync(wv.ptr, voxels, n * VX_CHUNK_VOLUME, cudaMemcpyHostToDevice, ctx->stream));
-    if (n && neighbors) VX_CUDA(ctx, cudaMemcpyAsync(wn.ptr, neighbors, n * 6 * sizeof(int32_t), cudaMemcpyHostToDevice, ctx->stream));
-    if (n && uniform_flags) VX_CUDA(ctx, cudaMemcpyAsync(wf.ptr, uniform_flags, n, cudaMemcpyHostToDevice, ctx->stream));
-    else if (n) VX_CUDA(ctx, cudaMemsetAsync(wf.ptr, 0, n, ctx->stream));
-    if (n && positions) VX_CUDA(ctx, cudaMemcpyAsync(ctx->tmp_d.ptr, positions, n * 3 * sizeof(int32_t), cudaMemcpyHostToDevice, ctx->stream));
-    int rc = vx_mesh_chunks_device(ctx, wv.as<uint8_t>(), positions ? ctx->tmp_d.as<int32_t>() : nullptr,
-                                   neighbors ? wn.as<int32_t>() : nullptr, wf.as<uint8_t>(), n_chunks, out);
-    if (rc != VX_OK) {
-        wv.release(); wn.release(); wf.release();
-        return rc;
+    BatchPtr b;
+    const int rc = new_batch(ctx, n_chunks, first_cap_quads(n_chunks), ALL_ARRAYS, b);
+    if (rc != VX_OK) return rc;
+    if (n) {
+        VX_CUDA(ctx, cudaMemcpyAsync(b->world_voxels.ptr, voxels, n * VX_CHUNK_VOLUME, cudaMemcpyHostToDevice, ctx->stream));
+        if (neighbors) VX_CUDA(ctx, cudaMemcpyAsync(b->world_neighbors.ptr, neighbors, n * 6 * sizeof(int32_t), cudaMemcpyHostToDevice, ctx->stream));
+        if (uniform_flags) VX_CUDA(ctx, cudaMemcpyAsync(b->world_flags.ptr, uniform_flags, n, cudaMemcpyHostToDevice, ctx->stream));
+        else VX_CUDA(ctx, cudaMemsetAsync(b->world_flags.ptr, 0, n, ctx->stream));
+        if (positions) VX_CUDA(ctx, cudaMemcpyAsync(b->positions.ptr, positions, n * 3 * sizeof(int32_t), cudaMemcpyHostToDevice, ctx->stream));
+        else VX_CUDA(ctx, cudaMemsetAsync(b->positions.ptr, 0, n * 3 * sizeof(int32_t), ctx->stream));
     }
-    VxMeshBatch *b = *out;
-    b->world_voxels = wv;
-    b->world_neighbors = wn;
-    b->world_flags = wf;
     b->owns_world = true;
     b->has_neighbors = neighbors != nullptr;
-    b->has_flags = true;
     if (neighbors) b->host_neighbors.assign(neighbors, neighbors + n * 6);
-    return VX_OK;
+    return mesh_new_batch(ctx, b, world_input(b.get()), nullptr, out);
 }
 
 int vx_mesh_batch_update(VxContext *ctx, VxMeshBatch *b, const int32_t *chunk_ids, int32_t n_ids, const uint8_t *voxels,
@@ -846,18 +951,14 @@ int vx_mesh_batch_update(VxContext *ctx, VxMeshBatch *b, const int32_t *chunk_id
     if (n_ids == 0) return VX_OK;
     VX_CUDA(ctx, cudaSetDevice(ctx->device));
     // edited chunks + the neighbours whose border faces they can change (main.rs:225-280 invalidates the same six)
-    std::vector<int32_t> list;
-    std::vector<uint8_t> seen((size_t)b->n_chunks, 0);
-    for (int32_t i = 0; i < n_ids; ++i) {
-        const int32_t c = chunk_ids[i];
+    std::vector<int32_t> ids(chunk_ids, chunk_ids + n_ids);
+    for (const int32_t c : ids)
         if (c < 0 || c >= b->n_chunks) return vx_fail(ctx, VX_ERR_INVALID, "vx_mesh_batch_update: chunk id out of range");
-        if (!seen[c]) { seen[c] = 1; list.push_back(c); }
-    }
     if (b->has_neighbors)
         for (int32_t i = 0; i < n_ids; ++i)
             for (int f = 0; f < 6; ++f) {
                 const int32_t nb = b->host_neighbors[(size_t)chunk_ids[i] * 6 + f];
-                if (nb >= 0 && nb < b->n_chunks && !seen[nb]) { seen[nb] = 1; list.push_back(nb); }
+                if (nb >= 0 && nb < b->n_chunks) ids.push_back(nb);
             }
     // new voxel data / uniform flags of the edited chunks into the world copy
     for (int32_t i = 0; i < n_ids; ++i) {
@@ -866,64 +967,32 @@ int vx_mesh_batch_update(VxContext *ctx, VxMeshBatch *b, const int32_t *chunk_id
         const uint8_t uf = uniform_flags ? uniform_flags[i] : 0;
         VX_CUDA(ctx, cudaMemsetAsync(b->world_flags.as<uint8_t>() + chunk_ids[i], uf, 1, ctx->stream));
     }
+    const std::vector<int32_t> list = unique_ids(ids, b->n_chunks);
     if (n_remeshed) *n_remeshed = (int32_t)list.size();
-    const uint8_t *d_vox = b->world_voxels.as<uint8_t>();
-    const int32_t *d_nb = b->has_neighbors ? b->world_neighbors.as<int32_t>() : nullptr;
-    const uint8_t *d_uf = b->world_flags.as<uint8_t>();
-    // room behind the live end of the quad stream?  (typical chunk: a few hundred quads; 4096 each is a generous
-    // bound that the overflow flag backs up.)  If not, or if an append overflows, re-mesh the whole world from
-    // scratch, which also drops the dead space.
-    VxMeshBatchInfo info;
-    int rc = vx_mesh_batch_info(ctx, b, &info);
-    if (rc != VX_OK) return rc;
-    bool full = info.total_quads + (int64_t)list.size() * 4096 > b->cap_quads;
-    if (!full) {
-        VX_CUDA(ctx, b->update_ids.reserve(sizeof(int32_t) * list.size()));
-        VX_CUDA(ctx, cudaMemcpyAsync(b->update_ids.ptr, list.data(), sizeof(int32_t) * list.size(), cudaMemcpyHostToDevice, ctx->stream));
-        rc = run_mesher(ctx, d_vox, d_nb, d_uf, b, false, b->update_ids.as<int32_t>(), b->n_chunks, true, (int32_t)list.size());
-        if (rc != VX_OK) return rc;
-        unsigned long long h[4];
-        VX_CUDA(ctx, cudaMemcpyAsync(h, b->cursor.ptr, sizeof(h), cudaMemcpyDeviceToHost, ctx->stream));
-        VX_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-        if (h[2]) full = true;
-        else b->total_quads = (int64_t)h[0]; // length of the stream, dead space included
-    }
-    if (full) {
-        if (b->cap_quads < info.total_quads + (int64_t)list.size() * 4096) { // also make room for the next updates
-            const int64_t want = info.total_quads * 2 + (int64_t)list.size() * 4096;
-            VX_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-            VX_CUDA(ctx, b->quads.reserve(3 * (size_t)want + 16));
-            b->cap_quads = want;
-        }
-        rc = run_mesher(ctx, d_vox, d_nb, d_uf, b, true);
-        if (rc != VX_OK) return rc;
-    }
-    b->n_meshes = -1; // recounted on demand
-    return VX_OK;
+    return remesh_listed(ctx, b, list);
 }
 
 int vx_mesh_batch_info(VxContext *ctx, const VxMeshBatch *b, VxMeshBatchInfo *info) {
     if (!ctx || !b || !info) return vx_fail(ctx, VX_ERR_INVALID, "vx_mesh_batch_info: bad argument");
-    VxMeshBatch *mb = const_cast<VxMeshBatch *>(b);
-    if (mb->total_quads < 0) {
-        unsigned long long h[4];
-        VX_CUDA(ctx, cudaMemcpyAsync(h, mb->cursor.ptr, sizeof(h), cudaMemcpyDeviceToHost, ctx->stream));
-        VX_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-        if (h[2]) return vx_fail(ctx, VX_ERR_CAPACITY, "remesh overflowed the batch quad stream");
-        mb->total_quads = (int64_t)h[0];
-        mb->n_meshes = (int32_t)h[1];
+    if (b->total_quads < 0) {
+        MeshCursor h;
+        const int rc = read_cursor(ctx, b, h);
+        if (rc != VX_OK) return rc;
+        if (h.overflow) return vx_fail(ctx, VX_ERR_CAPACITY, "remesh overflowed the batch quad stream");
+        b->total_quads = (int64_t)h.quads;
+        b->n_meshes = (int32_t)h.meshes;
     }
-    if (mb->n_meshes < 0) { // after an in-place update: count has_mesh
+    if (b->n_meshes < 0) { // after an in-place update: count has_mesh
         std::vector<uint8_t> hm((size_t)b->n_chunks);
         if (b->n_chunks) VX_CUDA(ctx, cudaMemcpyAsync(hm.data(), b->has_mesh.ptr, (size_t)b->n_chunks, cudaMemcpyDeviceToHost, ctx->stream));
         VX_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
         int32_t nm = 0;
         for (uint8_t v : hm) nm += v ? 1 : 0;
-        mb->n_meshes = nm;
+        b->n_meshes = nm;
     }
     info->n_chunks = b->n_chunks;
-    info->n_meshes = mb->n_meshes;
-    info->total_quads = mb->total_quads;
+    info->n_meshes = b->n_meshes;
+    info->total_quads = b->total_quads;
     return VX_OK;
 }
 
@@ -949,8 +1018,8 @@ int vx_mesh_batch_download(VxContext *ctx, const VxMeshBatch *b, uint8_t *quads,
     if (quads && info.total_quads) VX_CUDA(ctx, cudaMemcpyAsync(quads, b->quads.ptr, 3 * (size_t)info.total_quads, cudaMemcpyDeviceToHost, ctx->stream));
     if (quad_base && n) VX_CUDA(ctx, cudaMemcpyAsync(quad_base, b->quad_base.ptr, 4 * n, cudaMemcpyDeviceToHost, ctx->stream));
     if (quad_count && n) VX_CUDA(ctx, cudaMemcpyAsync(quad_count, b->quad_count.ptr, 4 * n, cudaMemcpyDeviceToHost, ctx->stream));
-    if (slice_offsets && n) VX_CUDA(ctx, cudaMemcpyAsync(slice_offsets, b->slice_offsets.ptr, 4 * 198 * n, cudaMemcpyDeviceToHost, ctx->stream));
-    if (face_aabb && n) VX_CUDA(ctx, cudaMemcpyAsync(face_aabb, b->face_aabb.ptr, 4 * 36 * n, cudaMemcpyDeviceToHost, ctx->stream));
+    if (slice_offsets && n) VX_CUDA(ctx, cudaMemcpyAsync(slice_offsets, b->slice_offsets.ptr, 4 * SLICE_ROW * n, cudaMemcpyDeviceToHost, ctx->stream));
+    if (face_aabb && n) VX_CUDA(ctx, cudaMemcpyAsync(face_aabb, b->face_aabb.ptr, 4 * AABB_ROW * n, cudaMemcpyDeviceToHost, ctx->stream));
     if (has_mesh && n) VX_CUDA(ctx, cudaMemcpyAsync(has_mesh, b->has_mesh.ptr, n, cudaMemcpyDeviceToHost, ctx->stream));
     VX_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
     return VX_OK;
@@ -963,30 +1032,27 @@ int vx_mesh_batch_upload(VxContext *ctx, const uint8_t *quads, int64_t total_qua
     if (n_chunks > 0 && (!quad_base || !quad_count || !slice_offsets || !face_aabb || !has_mesh || !positions))
         return vx_fail(ctx, VX_ERR_INVALID, "vx_mesh_batch_upload: null array");
     VX_CUDA(ctx, cudaSetDevice(ctx->device));
-    VxMeshBatch *b = new VxMeshBatch();
-    int rc = batch_alloc(ctx, b, n_chunks, total_quads > 0 ? total_quads : 1);
-    if (rc != VX_OK) { vx_mesh_batch_release(ctx, b); return rc; }
+    BatchPtr b;
+    int rc = new_batch(ctx, n_chunks, total_quads > 0 ? total_quads : 1, MESH_ARRAYS, b);
+    if (rc != VX_OK) return rc;
     const size_t n = (size_t)n_chunks;
-    cudaError_t e = cudaSuccess;
-    auto up = [&](void *dst, const void *src, size_t bytes) {
-        if (e == cudaSuccess && bytes) e = cudaMemcpyAsync(dst, src, bytes, cudaMemcpyHostToDevice, ctx->stream);
+    auto up = [&](void *dst, const void *src, size_t bytes) -> cudaError_t {
+        return bytes ? cudaMemcpyAsync(dst, src, bytes, cudaMemcpyHostToDevice, ctx->stream) : cudaSuccess;
     };
-    up(b->quads.ptr, quads, 3 * (size_t)total_quads);
-    up(b->quad_base.ptr, quad_base, 4 * n);
-    up(b->quad_count.ptr, quad_count, 4 * n);
-    up(b->slice_offsets.ptr, slice_offsets, 4 * 198 * n);
-    up(b->face_aabb.ptr, face_aabb, 4 * 36 * n);
-    up(b->has_mesh.ptr, has_mesh, n);
-    up(b->positions.ptr, positions, 12 * n);
+    VX_CUDA(ctx, up(b->quads.ptr, quads, 3 * (size_t)total_quads));
+    VX_CUDA(ctx, up(b->quad_base.ptr, quad_base, 4 * n));
+    VX_CUDA(ctx, up(b->quad_count.ptr, quad_count, 4 * n));
+    VX_CUDA(ctx, up(b->slice_offsets.ptr, slice_offsets, 4 * SLICE_ROW * n));
+    VX_CUDA(ctx, up(b->face_aabb.ptr, face_aabb, 4 * AABB_ROW * n));
+    VX_CUDA(ctx, up(b->has_mesh.ptr, has_mesh, n));
+    VX_CUDA(ctx, up(b->positions.ptr, positions, 12 * n));
     int32_t nm = 0;
     for (size_t i = 0; i < n; ++i) nm += has_mesh[i] ? 1 : 0;
-    unsigned long long h[4] = {(unsigned long long)total_quads, (unsigned long long)nm, 0, 0};
-    up(b->cursor.ptr, h, sizeof(h));
-    if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
-    if (e != cudaSuccess) { vx_mesh_batch_release(ctx, b); return vx_cuda_fail(ctx, e, "upload", __FILE__, __LINE__); }
+    rc = write_cursor(ctx, b.get(), MeshCursor{(unsigned long long)total_quads, (unsigned long long)nm, 0ull, 0ull});
+    if (rc != VX_OK) return rc;
     b->total_quads = total_quads;
     b->n_meshes = nm;
-    *out = b;
+    *out = b.release();
     return VX_OK;
 }
 
@@ -1004,8 +1070,8 @@ int vx_shard_layout(int32_t rows_per_rank, int64_t max_shard_quads, VxShardLayou
     out->rows_per_rank = rows_per_rank;
     out->off_quad_base = o; o = up16(o + 4 * rows);
     out->off_quad_count = o; o = up16(o + 4 * rows);
-    out->off_slice_offsets = o; o = up16(o + 4 * 198 * rows);
-    out->off_face_aabb = o; o = up16(o + 4 * 36 * rows);
+    out->off_slice_offsets = o; o = up16(o + 4 * SLICE_ROW * rows);
+    out->off_face_aabb = o; o = up16(o + 4 * AABB_ROW * rows);
     out->off_has_mesh = o; o = up16(o + rows);
     o += 16; // block[off_quads - 16 .. off_quads - 8): u64 quad total of the shard (vx_mesh_shard_pack_async)
     out->off_quads = o; o = up16(o + 3 * max_shard_quads);
@@ -1021,16 +1087,9 @@ int vx_mesh_shard_pack(VxContext *ctx, const VxMeshBatch *shard, const VxShardLa
     int rc = vx_mesh_batch_info(ctx, shard, &info);
     if (rc != VX_OK) return rc;
     if (info.total_quads > L->quads_capacity) return vx_fail(ctx, VX_ERR_CAPACITY, "shard has more quads than the layout holds");
-    const size_t n = (size_t)shard->n_chunks;
-    auto cp = [&](int64_t off, const void *src, size_t bytes) -> cudaError_t {
-        return bytes ? cudaMemcpyAsync(d_block + off, src, bytes, cudaMemcpyDeviceToDevice, ctx->stream) : cudaSuccess;
-    };
-    VX_CUDA(ctx, cp(L->off_quad_base, shard->quad_base.ptr, 4 * n));
-    VX_CUDA(ctx, cp(L->off_quad_count, shard->quad_count.ptr, 4 * n));
-    VX_CUDA(ctx, cp(L->off_slice_offsets, shard->slice_offsets.ptr, 4 * 198 * n));
-    VX_CUDA(ctx, cp(L->off_face_aabb, shard->face_aabb.ptr, 4 * 36 * n));
-    VX_CUDA(ctx, cp(L->off_has_mesh, shard->has_mesh.ptr, n));
-    VX_CUDA(ctx, cp(L->off_quads, shard->quads.ptr, 3 * (size_t)info.total_quads));
+    rc = pack_rows(ctx, shard, L, d_block);
+    if (rc != VX_OK) return rc;
+    VX_CUDA(ctx, to_block(ctx, d_block, L->off_quads, shard->quads.ptr, 3 * (size_t)info.total_quads));
     return VX_OK;
 }
 
@@ -1049,41 +1108,23 @@ int vx_mesh_batch_assemble_shards(VxContext *ctx, int32_t n_chunks, int32_t worl
         total += shard_quads[r];
     }
     if (total >= (int64_t)1 << 32) return vx_fail(ctx, VX_ERR_CAPACITY, "more than 2^32 quads in one batch");
-    VxMeshBatch *b = *batch_inout;
-    const bool fresh = b == nullptr;
-    if (!fresh && b->n_chunks != n_chunks) return vx_fail(ctx, VX_ERR_INVALID, "batch was created for another chunk count");
-    if (fresh) {
-        b = new VxMeshBatch();
-        int rc = batch_alloc(ctx, b, n_chunks, total > 0 ? total + total / 8 : 1);
-        if (rc != VX_OK) { vx_mesh_batch_release(ctx, b); return rc; }
-    } else if (total > b->cap_quads) {
-        VX_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-        VX_CUDA(ctx, b->quads.reserve(3 * (size_t)(total + total / 8) + 16));
-        b->cap_quads = total + total / 8;
-    }
-    cudaError_t e = cudaSuccess;
+    BatchPtr fresh;
+    const int rc = assemble_target(ctx, batch_inout, n_chunks, total, total + total / 8, d_positions, fresh);
+    if (rc != VX_OK) return rc;
+    VxMeshBatch *b = fresh ? fresh.get() : *batch_inout;
     if (n_chunks > 0) {
-        if (d_positions) e = cudaMemcpyAsync(b->positions.ptr, d_positions, sizeof(int32_t) * 3 * (size_t)n_chunks, cudaMemcpyDeviceToDevice, ctx->stream);
-        else if (fresh) e = cudaMemsetAsync(b->positions.ptr, 0, sizeof(int32_t) * 3 * (size_t)n_chunks, ctx->stream);
-        if (e == cudaSuccess) {
-            assemble_shards_kernel<<<n_chunks, 64, 0, ctx->stream>>>(n_chunks, world, so, d_blocks, *L, b->quad_base.as<uint32_t>(), b->quad_count.as<uint32_t>(),
-                                                                     b->slice_offsets.as<uint32_t>(), b->face_aabb.as<int32_t>(), b->has_mesh.as<uint8_t>(),
-                                                                     b->cursor.as<unsigned long long>(), (unsigned long long)total);
-            ctx->launches++;
-            e = cudaGetLastError();
-        }
+        assemble_shards_kernel<<<n_chunks, 64, 0, ctx->stream>>>(n_chunks, world, so, d_blocks, *L, b->quad_base.as<uint32_t>(), b->quad_count.as<uint32_t>(),
+                                                                 b->slice_offsets.as<uint32_t>(), b->face_aabb.as<int32_t>(), b->has_mesh.as<uint8_t>(),
+                                                                 b->cursor.as<MeshCursor>(), (unsigned long long)total);
+        VX_CHECK_LAUNCH(ctx);
     }
-    for (int r = 0; r < world && e == cudaSuccess; ++r)
+    for (int r = 0; r < world; ++r)
         if (shard_quads[r])
-            e = cudaMemcpyAsync(b->quads.as<uint8_t>() + 3 * (size_t)so.off[r], d_blocks + (size_t)r * (size_t)L->rank_stride + L->off_quads,
-                                3 * (size_t)shard_quads[r], cudaMemcpyDeviceToDevice, ctx->stream);
-    if (e != cudaSuccess) {
-        if (fresh) vx_mesh_batch_release(ctx, b);
-        return vx_cuda_fail(ctx, e, "assemble shards", __FILE__, __LINE__);
-    }
+            VX_CUDA(ctx, cudaMemcpyAsync(b->quads.as<uint8_t>() + 3 * (size_t)so.off[r], d_blocks + (size_t)r * (size_t)L->rank_stride + L->off_quads,
+                                         3 * (size_t)shard_quads[r], cudaMemcpyDeviceToDevice, ctx->stream));
     b->total_quads = total;
     b->n_meshes = -1; // counted on demand (vx_mesh_batch_info)
-    *batch_inout = b;
+    if (fresh) *batch_inout = fresh.release();
     return VX_OK;
 }
 
@@ -1094,18 +1135,11 @@ int vx_mesh_batch_assemble_shards(VxContext *ctx, int32_t n_chunks, int32_t worl
 int vx_mesh_shard_pack_async(VxContext *ctx, const VxMeshBatch *shard, const VxShardLayout *L, uint8_t *d_block) {
     if (!ctx || !shard || !L || !d_block || shard->n_chunks > L->rows_per_rank) return vx_fail(ctx, VX_ERR_INVALID, "vx_mesh_shard_pack_async: bad argument");
     VX_CUDA(ctx, cudaSetDevice(ctx->device));
-    const size_t n = (size_t)shard->n_chunks;
-    auto cp = [&](int64_t off, const void *src, size_t bytes) -> cudaError_t {
-        return bytes ? cudaMemcpyAsync(d_block + off, src, bytes, cudaMemcpyDeviceToDevice, ctx->stream) : cudaSuccess;
-    };
-    VX_CUDA(ctx, cp(L->off_quad_base, shard->quad_base.ptr, 4 * n));
-    VX_CUDA(ctx, cp(L->off_quad_count, shard->quad_count.ptr, 4 * n));
-    VX_CUDA(ctx, cp(L->off_slice_offsets, shard->slice_offsets.ptr, 4 * 198 * n));
-    VX_CUDA(ctx, cp(L->off_face_aabb, shard->face_aabb.ptr, 4 * 36 * n));
-    VX_CUDA(ctx, cp(L->off_has_mesh, shard->has_mesh.ptr, n));
+    const int rc = pack_rows(ctx, shard, L, d_block);
+    if (rc != VX_OK) return rc;
     const int64_t q = shard->cap_quads < L->quads_capacity ? shard->cap_quads : L->quads_capacity;
-    VX_CUDA(ctx, cp(L->off_quads, shard->quads.ptr, 3 * (size_t)(q > 0 ? q : 0)));
-    VX_CUDA(ctx, cp(L->off_quads - 16, shard->cursor.ptr, sizeof(unsigned long long)));
+    VX_CUDA(ctx, to_block(ctx, d_block, L->off_quads, shard->quads.ptr, 3 * (size_t)(q > 0 ? q : 0)));
+    VX_CUDA(ctx, to_block(ctx, d_block, L->off_quads - 16, shard->cursor.as<uint8_t>() + offsetof(MeshCursor, quads), sizeof(unsigned long long)));
     return VX_OK;
 }
 
@@ -1116,56 +1150,38 @@ int vx_mesh_batch_assemble_shards_async(VxContext *ctx, int32_t n_chunks, int32_
     VX_CUDA(ctx, cudaSetDevice(ctx->device));
     const int64_t bound = (int64_t)world * L->quads_capacity; // the assembled stream can never need more
     if (bound >= (int64_t)1 << 32) return vx_fail(ctx, VX_ERR_CAPACITY, "more than 2^32 quads in one batch");
-    VxMeshBatch *b = *batch_inout;
-    const bool fresh = b == nullptr;
-    if (!fresh && b->n_chunks != n_chunks) return vx_fail(ctx, VX_ERR_INVALID, "batch was created for another chunk count");
-    if (fresh) {
-        b = new VxMeshBatch();
-        int rc = batch_alloc(ctx, b, n_chunks, bound > 0 ? bound : 1);
-        if (rc != VX_OK) { vx_mesh_batch_release(ctx, b); return rc; }
-    } else if (bound > b->cap_quads) {
-        VX_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-        VX_CUDA(ctx, b->quads.reserve(3 * (size_t)bound + 16));
-        b->cap_quads = bound;
-    }
-    cudaError_t e = ctx->tmp_d.reserve(sizeof(uint32_t) * 128);
-    if (e == cudaSuccess && n_chunks > 0) {
-        if (d_positions) e = cudaMemcpyAsync(b->positions.ptr, d_positions, sizeof(int32_t) * 3 * (size_t)n_chunks, cudaMemcpyDeviceToDevice, ctx->stream);
-        else if (fresh) e = cudaMemsetAsync(b->positions.ptr, 0, sizeof(int32_t) * 3 * (size_t)n_chunks, ctx->stream);
-    }
-    if (e == cudaSuccess) {
-        uint32_t *d_off = ctx->tmp_d.as<uint32_t>();
-        shard_offsets_kernel<<<1, 32, 0, ctx->stream>>>(world, d_blocks, *L, d_off, b->cursor.as<unsigned long long>(), (unsigned long long)b->cap_quads);
-        ctx->launches++;
-        if (n_chunks > 0) {
-            ShardOffsets none;
-            memset(&none, 0, sizeof(none));
-            assemble_shards_kernel<<<n_chunks, 64, 0, ctx->stream>>>(n_chunks, world, none, d_blocks, *L, b->quad_base.as<uint32_t>(), b->quad_count.as<uint32_t>(),
-                                                                     b->slice_offsets.as<uint32_t>(), b->face_aabb.as<int32_t>(), b->has_mesh.as<uint8_t>(),
-                                                                     b->cursor.as<unsigned long long>(), 0ull, d_off);
-            ctx->launches++;
-            const int per_rank = (int)((L->quads_capacity + 255) / 256 < 1 ? 1 : ((L->quads_capacity + 255) / 256 > 1024 ? 1024 : (L->quads_capacity + 255) / 256));
-            copy_shard_quads_kernel<<<dim3(per_rank, world), 256, 0, ctx->stream>>>(d_blocks, *L, d_off, b->quads.as<uint8_t>(), (unsigned long long)b->cap_quads);
-            ctx->launches++;
-        }
-        e = cudaGetLastError();
-    }
-    if (e != cudaSuccess) {
-        if (fresh) vx_mesh_batch_release(ctx, b);
-        return vx_cuda_fail(ctx, e, "assemble shards (async)", __FILE__, __LINE__);
+    BatchPtr fresh;
+    const int rc = assemble_target(ctx, batch_inout, n_chunks, bound, bound, d_positions, fresh);
+    if (rc != VX_OK) return rc;
+    VxMeshBatch *b = fresh ? fresh.get() : *batch_inout;
+    VX_CUDA(ctx, ctx->tmp_d.reserve(sizeof(uint32_t) * 128));
+    uint32_t *d_off = ctx->tmp_d.as<uint32_t>();
+    shard_offsets_kernel<<<1, 32, 0, ctx->stream>>>(world, d_blocks, *L, d_off, b->cursor.as<MeshCursor>(), (unsigned long long)b->cap_quads);
+    VX_CHECK_LAUNCH(ctx);
+    if (n_chunks > 0) {
+        ShardOffsets none;
+        memset(&none, 0, sizeof(none));
+        assemble_shards_kernel<<<n_chunks, 64, 0, ctx->stream>>>(n_chunks, world, none, d_blocks, *L, b->quad_base.as<uint32_t>(), b->quad_count.as<uint32_t>(),
+                                                                 b->slice_offsets.as<uint32_t>(), b->face_aabb.as<int32_t>(), b->has_mesh.as<uint8_t>(),
+                                                                 b->cursor.as<MeshCursor>(), 0ull, d_off);
+        VX_CHECK_LAUNCH(ctx);
+        const int per_rank = (int)((L->quads_capacity + 255) / 256 < 1 ? 1 : ((L->quads_capacity + 255) / 256 > 1024 ? 1024 : (L->quads_capacity + 255) / 256));
+        copy_shard_quads_kernel<<<dim3(per_rank, world), 256, 0, ctx->stream>>>(d_blocks, *L, d_off, b->quads.as<uint8_t>(), (unsigned long long)b->cap_quads);
+        VX_CHECK_LAUNCH(ctx);
     }
     b->total_quads = -1; // read from the device on demand (vx_mesh_batch_info), together with the overflow flag
     b->n_meshes = -1;
-    *batch_inout = b;
+    if (fresh) *batch_inout = fresh.release();
     return VX_OK;
 }
 
 void vx_mesh_batch_release(VxContext *ctx, VxMeshBatch *b) {
     if (!b) return;
     if (ctx) cudaSetDevice(ctx->device);
-    b->quads.release(); b->quad_base.release(); b->quad_count.release(); b->slice_offsets.release();
-    b->face_aabb.release(); b->has_mesh.release(); b->positions.release(); b->cursor.release();
-    b->world_voxels.release(); b->world_neighbors.release(); b->world_flags.release(); b->update_ids.release();
+    for (const ChunkArray &c : CHUNK_ARRAYS) (b->*c.buf).release();
+    b->quads.release();
+    b->cursor.release();
+    b->update_ids.release();
     delete b;
 }
 
@@ -1193,37 +1209,20 @@ int vx_greedy_mesh_slices(VxContext *ctx, const uint32_t *masks, int32_t n_slice
 int vx_world_batch_create(VxContext *ctx, int32_t capacity, VxMeshBatch **out) {
     if (!ctx || !out || capacity <= 0) return vx_fail(ctx, VX_ERR_INVALID, "vx_world_batch_create: bad argument");
     VX_CUDA(ctx, cudaSetDevice(ctx->device));
-    VxMeshBatch *b = new VxMeshBatch();
     const size_t n = (size_t)capacity;
-    int rc = batch_alloc(ctx, b, capacity, (int64_t)capacity * 512);
-    cudaError_t e = cudaSuccess;
-    if (rc == VX_OK) e = b->world_voxels.reserve(n * VX_CHUNK_VOLUME + 16);
-    if (rc == VX_OK && e == cudaSuccess) e = b->world_neighbors.reserve(n * 6 * sizeof(int32_t) + 16);
-    if (rc == VX_OK && e == cudaSuccess) e = b->world_flags.reserve(n + 16);
-    if (rc == VX_OK && e == cudaSuccess) { // every slot starts as an absent chunk: no neighbours, "uniform air", no mesh
-        cudaMemsetAsync(b->world_neighbors.ptr, 0xFF, n * 6 * sizeof(int32_t), ctx->stream); // -1 = VX_NBR_NONE
-        cudaMemsetAsync(b->world_flags.ptr, 1, n, ctx->stream);
-        cudaMemsetAsync(b->positions.ptr, 0, sizeof(int32_t) * 3 * n, ctx->stream);
-        cudaMemsetAsync(b->has_mesh.ptr, 0, n, ctx->stream);
-        cudaMemsetAsync(b->quad_count.ptr, 0, sizeof(uint32_t) * n, ctx->stream);
-        cudaMemsetAsync(b->quad_base.ptr, 0, sizeof(uint32_t) * n, ctx->stream);
-        cudaMemsetAsync(b->slice_offsets.ptr, 0, sizeof(uint32_t) * 198 * n, ctx->stream);
-        cudaMemsetAsync(b->face_aabb.ptr, 0, sizeof(int32_t) * 36 * n, ctx->stream);
-        cudaMemsetAsync(b->cursor.ptr, 0, sizeof(unsigned long long) * 4, ctx->stream);
-        e = cudaStreamSynchronize(ctx->stream);
-    }
-    if (rc == VX_OK && e != cudaSuccess) rc = vx_cuda_fail(ctx, e, "vx_world_batch_create", __FILE__, __LINE__);
-    if (rc != VX_OK) {
-        vx_mesh_batch_release(ctx, b);
-        return rc;
-    }
+    BatchPtr b;
+    int rc = new_batch(ctx, capacity, first_cap_quads(capacity), ALL_ARRAYS, b);
+    if (rc != VX_OK) return rc;
+    for (const ChunkArray &c : CHUNK_ARRAYS) // every slot starts as an absent chunk: no neighbours, "uniform air", no mesh
+        VX_CUDA(ctx, cudaMemsetAsync((b.get()->*c.buf).ptr, c.absent, c.row_bytes * n, ctx->stream));
+    rc = write_cursor(ctx, b.get(), MeshCursor{});
+    if (rc != VX_OK) return rc;
     b->owns_world = true;
     b->has_neighbors = true;
-    b->has_flags = true;
     b->host_neighbors.assign(n * 6, -1);
     b->total_quads = 0;
     b->n_meshes = 0;
-    *out = b;
+    *out = b.release();
     return VX_OK;
 }
 
@@ -1239,7 +1238,7 @@ int vx_world_batch_grow(VxContext *ctx, VxMeshBatch *b, int32_t new_capacity) {
     const size_t n0 = (size_t)b->n_chunks, n1 = (size_t)new_capacity;
     auto grow = [&](VxDeviceBuffer &buf, size_t per, int fill) -> cudaError_t {
         VxDeviceBuffer fresh;
-        cudaError_t e = fresh.reserve(n1 * per + 16);
+        cudaError_t e = fresh.reserve(n1 * per);
         if (e != cudaSuccess) return e;
         e = cudaMemcpyAsync(fresh.ptr, buf.ptr, n0 * per, cudaMemcpyDeviceToDevice, ctx->stream);
         if (e == cudaSuccess) e = cudaMemsetAsync(static_cast<uint8_t *>(fresh.ptr) + n0 * per, fill, (n1 - n0) * per, ctx->stream);
@@ -1252,15 +1251,7 @@ int vx_world_batch_grow(VxContext *ctx, VxMeshBatch *b, int32_t new_capacity) {
         buf = fresh;
         return cudaSuccess;
     };
-    VX_CUDA(ctx, grow(b->world_voxels, VX_CHUNK_VOLUME, 0));
-    VX_CUDA(ctx, grow(b->world_neighbors, 6 * sizeof(int32_t), 0xFF)); // VX_NBR_NONE
-    VX_CUDA(ctx, grow(b->world_flags, 1, 1));                          // "uniform air": an absent chunk
-    VX_CUDA(ctx, grow(b->positions, 3 * sizeof(int32_t), 0));
-    VX_CUDA(ctx, grow(b->has_mesh, 1, 0));
-    VX_CUDA(ctx, grow(b->quad_count, sizeof(uint32_t), 0));
-    VX_CUDA(ctx, grow(b->quad_base, sizeof(uint32_t), 0));
-    VX_CUDA(ctx, grow(b->slice_offsets, 198 * sizeof(uint32_t), 0));
-    VX_CUDA(ctx, grow(b->face_aabb, 36 * sizeof(int32_t), 0));
+    for (const ChunkArray &c : CHUNK_ARRAYS) VX_CUDA(ctx, grow(b->*c.buf, c.row_bytes, c.absent));
     b->host_neighbors.resize(n1 * 6, -1);
     b->n_chunks = new_capacity;
     return VX_OK;
@@ -1337,11 +1328,7 @@ int vx_world_batch_remesh(VxContext *ctx, VxMeshBatch *b, const int32_t *slots, 
     int rc = world_check_slots(ctx, b, slots, n, "vx_world_batch_remesh: bad argument");
     if (rc != VX_OK || n == 0) return rc;
     VX_CUDA(ctx, cudaSetDevice(ctx->device));
-    std::vector<int32_t> list;
-    std::vector<uint8_t> seen((size_t)b->n_chunks, 0);
-    for (int32_t i = 0; i < n; ++i)
-        if (!seen[slots[i]]) { seen[slots[i]] = 1; list.push_back(slots[i]); }
-    return remesh_listed(ctx, b, list);
+    return remesh_listed(ctx, b, unique_ids(std::vector<int32_t>(slots, slots + n), b->n_chunks));
 }
 
 } // extern "C"

@@ -251,8 +251,8 @@ VX_API int vx_mesh_chunks(VxContext *ctx, const uint8_t *voxels, const int32_t *
  *   chunk_ids      n_ids edited chunks (indices into the batch)
  *   voxels         n_ids x 32768 new voxel data, uniform_flags n_ids (as vx_mesh_chunks) or NULL = all Varied
  * The edited chunks and the neighbours listed for them at creation are re-meshed in place (*n_remeshed of them); new
- * quads are appended to the quad stream, the replaced ones become dead space that the next full re-mesh (triggered
- * automatically when the stream runs out of room) drops.  Every other chunk's mesh is untouched. */
+ * quads are appended to the quad stream, the replaced ones become dead space.  When the stream runs out of room the
+ * live quads are compacted (copied, not re-meshed).  Every other chunk's mesh is untouched. */
 VX_API int vx_mesh_batch_update(VxContext *ctx, VxMeshBatch *batch, const int32_t *chunk_ids, int32_t n_ids, const uint8_t *voxels,
                          const uint8_t *uniform_flags, int32_t *n_remeshed);
 /* Same with all four arrays already resident on the context's device. */

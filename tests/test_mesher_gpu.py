@@ -243,7 +243,7 @@ def test_chunk_subset_meshing_matches_the_full_batch(ctx, ob):
 def test_incremental_update_matches_a_full_remesh(ctx, ob):
     """vx_mesh_batch_update (edit -> re-mesh the chunk and its six neighbours, main.rs:225-280): after every round of
     edits each chunk's mesh equals the oracle's mesh of the edited world, including the rounds where the quad stream
-    runs out of room and the batch falls back to a full re-mesh."""
+    runs out of room and its live quads are compacted."""
     import vx_scenes
     pos, world, p, v, nb = vx_scenes.terrain_scene(3)
     v = v.copy()
@@ -270,7 +270,7 @@ def test_incremental_update_matches_a_full_remesh(ctx, ob):
         assert ids.size <= nre <= 7 * ids.size
         info = batch.info()
         if info.total_quads < before:
-            fell_back = True  # the stream was rebuilt from scratch
+            fell_back = True  # the stream was compacted
         ref = ob.mesh_chunks(v, nb, None, p)
         got = batch.download()
         assert np.array_equal(got["quad_count"], ref.quad_count), rnd
@@ -286,7 +286,7 @@ def test_incremental_update_matches_a_full_remesh(ctx, ob):
     fresh = api.BinaryGreedyMesher.mesh_batch(v, p, nb, None, ctx)
     c2, d2, s2 = api.render_frame(fresh, vp, cam.position, cfg, view_distance=3, ctx=ctx)
     assert np.array_equal(c1, c2) and np.array_equal(d1.view(np.uint32), d2.view(np.uint32)) and np.array_equal(s1, s2)
-    print("fell back to a full re-mesh at least once:", fell_back)
+    print("compacted the quad stream at least once:", fell_back)
     fresh.release()
     batch.release()
     # a batch that does not own its world refuses the update
@@ -299,6 +299,37 @@ def test_incremental_update_matches_a_full_remesh(ctx, ob):
     with pytest.raises(api.VxError):
         b2.update(np.array([0], np.int32), v[:1])
     b2.release()
+
+
+def test_update_leaves_chunks_outside_its_list_untouched(ctx, ob):
+    """vx_mesh_batch_update re-meshes only the edited chunks and the neighbours listed for them, also when the quad stream
+    is full.  C lists E as its +X neighbour, E lists no neighbours: an edit of E's x = 0 plane changes the faces C would
+    get, but C is not in the list, so its mesh stays bit-identical (stale, like the reference's mesh cache)."""
+    C, E = 0, 1
+    c = kat.empty_chunk().reshape(32, 32, 32)  # [z][y][x]
+    c[4:20, 2:30, 31] = kat.STONE              # a wall on C's +X border
+    e = kat.empty_chunk().reshape(32, 32, 32)
+    e[10:12, 10:12, 10:12] = kat.DIRT
+    vox = np.stack([c.reshape(-1), e.reshape(-1), kat.chunk_single_voxel()])  # the third chunk is filler
+    nb = np.full((3, 6), -1, dtype=np.int32)
+    nb[C, 0] = E
+    batch = api.BinaryGreedyMesher.mesh_batch(vox, None, nb, None, ctx)
+    before = batch.download()
+    c_quads = batch.chunk_quads(C).copy()
+    new_e = e.copy()
+    new_e[:, :, 0] = kat.GRASS                 # E's x = 0 plane now hides C's wall
+    vox[E] = new_e.reshape(-1)
+    assert batch.update(np.array([E], np.int32), vox[E:E + 1]) == 1
+    ref = ob.mesh_chunks(vox, nb, None, None)
+    assert not np.array_equal(ref.chunk_quads(C).reshape(-1), c_quads.reshape(-1))  # a re-mesh of C would change it
+    got = batch.download()
+    assert np.array_equal(batch.chunk_quads(C), c_quads)
+    for k in ("quad_count", "slice_offsets", "face_aabb", "has_mesh"):
+        assert np.array_equal(got[k][C], before[k][C]), k
+    assert np.array_equal(batch.chunk_quads(E).reshape(-1), ref.chunk_quads(E).reshape(-1))
+    assert got["quad_count"][E] == ref.quad_count[E] and got["has_mesh"][E] == ref.has_mesh[E]
+    assert np.array_equal(got["slice_offsets"][E], ref.slice_offsets[E]) and np.array_equal(got["face_aabb"][E], ref.face_aabb[E])
+    batch.release()
 
 
 def test_device_terrain_generation_matches_the_oracle(ctx, ob):
