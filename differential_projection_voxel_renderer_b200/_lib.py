@@ -24,6 +24,11 @@ NBR_NONE = -1
 NBR_UNIFORM_AIR = -2
 NBR_UNIFORM_SOLID = -3
 
+RAY_HIT = 0
+RAY_MISS = 1
+RAY_LEFT_WORLD = 2
+RAY_INVALID = 3
+
 
 class VxError(RuntimeError):
     def __init__(self, code: int, msg: str):
@@ -76,6 +81,11 @@ class VxShardLayout(C.Structure):
     _fields_ = [("rank_stride", C.c_int64), ("off_quad_base", C.c_int64), ("off_quad_count", C.c_int64),
                 ("off_slice_offsets", C.c_int64), ("off_face_aabb", C.c_int64), ("off_has_mesh", C.c_int64),
                 ("off_quads", C.c_int64), ("quads_capacity", C.c_int64), ("rows_per_rank", C.c_int32), ("reserved", C.c_int32)]
+
+
+class VxRayHit(C.Structure):
+    _fields_ = [("status", C.c_int32), ("slot", C.c_int32), ("voxel", C.c_int32 * 3), ("face", C.c_int32), ("t", C.c_float),
+                ("block_type", C.c_uint8), ("pad", C.c_uint8 * 3)]
 
 
 class VxFrameStats(C.Structure):
@@ -135,6 +145,9 @@ PROTOTYPES = {
     "vx_world_batch_generate": (C.c_int, [_P, _P, _P, _I, _P, C.POINTER(VxTerrainParams), _P]),
     "vx_world_batch_unload": (C.c_int, [_P, _P, _P, _I]),
     "vx_world_batch_remesh": (C.c_int, [_P, _P, _P, _I]),
+    "vx_world_batch_set_blocks": (C.c_int, [_P, _P, _P, _P, _P, _I]),
+    "vx_world_raycast": (C.c_int, [_P, _P, _P, _P, _P, _I, C.c_float, _P]),
+    "vx_world_raycast_device": (C.c_int, [_P, _P, _P, _P, _P, _I, C.c_float, _P]),
     "vx_render_mesh_tiny_quads": (C.c_int, [_P, _P, _I, _P, C.POINTER(VxFrameConfig), _P, _I, _P, _P]),
     "vx_render_mesh_with_up": (C.c_int, [_P, _P, _I, _P, C.POINTER(VxFrameConfig), _P, _P, _P]),
     "vx_render_frame_macrotile": (C.c_int, [_P, _P, _P, _I, _P, C.POINTER(VxFrameConfig), _P, _P, _P, C.POINTER(_I)]),

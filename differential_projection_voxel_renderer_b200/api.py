@@ -594,6 +594,33 @@ def render_frame(batch: MeshBatch, view_proj, camera_position, cfg: VxFrameConfi
     return color_out, depth_out, (surv[:ns.value] if survivors_out is not None else surv[:ns.value].copy())
 
 
+# ---- picking (vx_world_raycast) ------------------------------------------------------------------------------------
+
+RAY_HIT_DTYPE = np.dtype([("status", "<i4"), ("slot", "<i4"), ("voxel", "<i4", (3,)), ("face", "<i4"), ("t", "<f4"),
+                          ("block_type", "u1"), ("pad", "u1", (3,))])  # VxRayHit, 32 bytes
+assert RAY_HIT_DTYPE.itemsize == C.sizeof(_lib.VxRayHit)
+
+
+def pixel_rays(view_proj, camera_position, pixels, width: int, height: int):
+    """Rays from the camera through pixel centres, for vx_world_raycast: origin = camera_position, direction = the pixel
+    centre (the rasterizer's convention: ndc.x = (px + 0.5) / W * 2 - 1, ndc.y = 1 - (py + 0.5) / H * 2) unprojected at the
+    far plane (ndc.z = 1) through the inverse view-projection, in float64, normalised, then rounded to f32.
+    pixels: (n, 2) (px, py).  Returns (origins (n, 3) f32, dirs (n, 3) f32)."""
+    m = np.asarray(view_proj, dtype=np.float32).reshape(4, 4).T.astype(np.float64)  # column-major -> row-major
+    px = np.asarray(pixels, dtype=np.float64).reshape(-1, 2)
+    n = px.shape[0]
+    ndc = np.empty((n, 4), dtype=np.float64)
+    ndc[:, 0] = (px[:, 0] + 0.5) / width * 2.0 - 1.0
+    ndc[:, 1] = 1.0 - (px[:, 1] + 0.5) / height * 2.0
+    ndc[:, 2] = 1.0
+    ndc[:, 3] = 1.0
+    far = ndc @ np.linalg.inv(m).T
+    cam = np.asarray(camera_position, dtype=np.float32).reshape(3)
+    d = far[:, :3] / far[:, 3:4] - cam.astype(np.float64)
+    d /= np.linalg.norm(d, axis=1, keepdims=True)
+    return np.repeat(cam.reshape(1, 3), n, axis=0), d.astype(np.float32)
+
+
 def hyper_pipeline_render(batch: MeshBatch, mesh_ids, view_proj, framebuffer: Framebuffer, ctx: Optional[Context] = None) -> int:
     """The Hyper-Pipeline for a list of meshes (vx_hyper_pipeline_render): face packets -> PacketPipeline
     (packet_pipeline.rs:69-142) -> span walker, into `framebuffer` (read-modify-write).  Returns the quads that passed the

@@ -24,6 +24,7 @@
 
 #include <cstddef>
 #include <memory>
+#include <unordered_set>
 #include <vector>
 
 namespace {
@@ -861,6 +862,26 @@ int remesh_listed(VxContext *ctx, VxMeshBatch *b, const std::vector<int32_t> &li
     return vx_fail(ctx, VX_ERR_CAPACITY, "world batch: quad stream overflow persisted");
 }
 
+// vx_world_batch_set_blocks, step 1: one CTA per edited slot.  A Uniform slot gets voxel rows of its block type and becomes
+// Varied, so that the edits of step 2 land in a complete chunk.
+constexpr int EDIT_THREADS = 256;
+__global__ void __launch_bounds__(EDIT_THREADS) materialize_uniform_kernel(uint8_t *voxels, uint8_t *flags, const int32_t *slots) {
+    const int32_t s = slots[blockIdx.x];
+    const uint8_t flag = flags[s];
+    if (flag == 0) return; // uniform across the CTA: no thread reaches the barrier
+    const uint32_t t = (uint32_t)(flag - 1) * 0x01010101u;
+    uint4 *row = reinterpret_cast<uint4 *>(voxels + (size_t)s * VX_CHUNK_VOLUME);
+    for (int k = threadIdx.x; k < VX_CHUNK_VOLUME / 16; k += EDIT_THREADS) row[k] = make_uint4(t, t, t, t);
+    __syncthreads(); // every thread has read the flag
+    if (threadIdx.x == 0) flags[s] = 0;
+}
+
+// step 2: one thread per edit; the host has removed repeated voxels, so no two threads store to the same byte
+__global__ void scatter_blocks_kernel(uint8_t *voxels, const int32_t *slot, const int32_t *index, const int32_t *type, int32_t n) {
+    const int32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < n) voxels[(size_t)slot[i] * VX_CHUNK_VOLUME + index[i]] = (uint8_t)type[i];
+}
+
 } // namespace
 
 extern "C" {
@@ -1329,6 +1350,45 @@ int vx_world_batch_remesh(VxContext *ctx, VxMeshBatch *b, const int32_t *slots, 
     if (rc != VX_OK || n == 0) return rc;
     VX_CUDA(ctx, cudaSetDevice(ctx->device));
     return remesh_listed(ctx, b, unique_ids(std::vector<int32_t>(slots, slots + n), b->n_chunks));
+}
+
+int vx_world_batch_set_blocks(VxContext *ctx, VxMeshBatch *b, const int32_t *slots, const int32_t *voxel_index, const uint8_t *block_types,
+                              int32_t n) {
+    int rc = world_check_slots(ctx, b, slots, n, "vx_world_batch_set_blocks: bad argument");
+    if (rc != VX_OK || n == 0) return rc;
+    if (!voxel_index || !block_types) return vx_fail(ctx, VX_ERR_INVALID, "vx_world_batch_set_blocks: bad argument");
+    for (int32_t i = 0; i < n; ++i) {
+        if (voxel_index[i] < 0 || voxel_index[i] >= VX_CHUNK_VOLUME) return vx_fail(ctx, VX_ERR_INVALID, "vx_world_batch_set_blocks: voxel index out of range");
+        if (block_types[i] > 3) return vx_fail(ctx, VX_ERR_INVALID, "vx_world_batch_set_blocks: block type out of range");
+    }
+    VX_CUDA(ctx, cudaSetDevice(ctx->device));
+    // last edit of a voxel wins: walk the list backwards and keep the first occurrence of each (slot, voxel)
+    std::vector<int32_t> es, ei, et;
+    std::unordered_set<int64_t> seen;
+    for (int32_t i = n - 1; i >= 0; --i)
+        if (seen.insert((int64_t)slots[i] * VX_CHUNK_VOLUME + voxel_index[i]).second) {
+            es.push_back(slots[i]);
+            ei.push_back(voxel_index[i]);
+            et.push_back(block_types[i]);
+        }
+    const std::vector<int32_t> touched = unique_ids(es, b->n_chunks);
+    const size_t m = touched.size(), k = es.size();
+    std::vector<int32_t> staged; // distinct slots, then slot, voxel index and type of each edit
+    staged.reserve(m + 3 * k);
+    staged.insert(staged.end(), touched.begin(), touched.end());
+    staged.insert(staged.end(), es.begin(), es.end());
+    staged.insert(staged.end(), ei.begin(), ei.end());
+    staged.insert(staged.end(), et.begin(), et.end());
+    VX_CUDA(ctx, ctx->tmp_a.reserve(sizeof(int32_t) * staged.size()));
+    int32_t *d = ctx->tmp_a.as<int32_t>();
+    VX_CUDA(ctx, cudaMemcpyAsync(d, staged.data(), sizeof(int32_t) * staged.size(), cudaMemcpyHostToDevice, ctx->stream));
+    materialize_uniform_kernel<<<(unsigned)m, EDIT_THREADS, 0, ctx->stream>>>(b->world_voxels.as<uint8_t>(), b->world_flags.as<uint8_t>(), d);
+    VX_CHECK_LAUNCH(ctx);
+    scatter_blocks_kernel<<<(unsigned)((k + 255) / 256), 256, 0, ctx->stream>>>(b->world_voxels.as<uint8_t>(), d + m, d + m + k, d + m + 2 * k,
+                                                                                  (int32_t)k);
+    VX_CHECK_LAUNCH(ctx);
+    VX_CUDA(ctx, cudaStreamSynchronize(ctx->stream)); // `staged` goes out of scope
+    return VX_OK;
 }
 
 } // extern "C"

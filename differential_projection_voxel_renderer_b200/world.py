@@ -13,7 +13,7 @@ from typing import Dict, Iterable, List, Optional, Tuple
 
 import numpy as np
 
-from . import api
+from . import _lib, api
 from ._lib import VxTerrainParams
 
 Pos = Tuple[int, int, int]
@@ -47,7 +47,8 @@ def sphere_capacity(view_distance: int) -> int:
 
 
 class _DeviceWorld:
-    """The five vx_world_batch_* calls; tests substitute a recorder for it to check the host logic without a GPU."""
+    """The vx_world_batch_* calls and vx_world_raycast; tests substitute a recorder for it to check the host logic without a
+    GPU."""
 
     def __init__(self, ctx: api.Context, capacity: int, terrain: VxTerrainParams):
         self.ctx = ctx
@@ -78,6 +79,16 @@ class _DeviceWorld:
     def remesh(self, slots: np.ndarray):
         self.ctx.check(self.ctx.lib.vx_world_batch_remesh(self.ctx.handle, self.batch.handle, api._p(slots), int(slots.size)))
 
+    def set_blocks(self, slots: np.ndarray, voxel_index: np.ndarray, block_types: np.ndarray):
+        self.ctx.check(self.ctx.lib.vx_world_batch_set_blocks(self.ctx.handle, self.batch.handle, api._p(slots), api._p(voxel_index),
+                                                              api._p(block_types), int(slots.size)))
+
+    def raycast(self, origins: np.ndarray, dirs: np.ndarray, start_slots: np.ndarray, max_t: float) -> np.ndarray:
+        hits = np.zeros(start_slots.size, dtype=api.RAY_HIT_DTYPE)
+        self.ctx.check(self.ctx.lib.vx_world_raycast(self.ctx.handle, self.batch.handle, api._p(origins), api._p(dirs), api._p(start_slots),
+                                                     int(start_slots.size), float(max_t), api._p(hits)))
+        return hits
+
 
 class World:
     """world.rs:30-215 with device-resident chunks: `chunks` maps a lattice position to its slot in the world batch."""
@@ -90,6 +101,9 @@ class World:
                                                                      terrain or api.terrain_params())
         self.chunks: Dict[Pos, int] = {}
         self.uniform_flags: Dict[Pos, int] = {}   # 0 Varied, 1 + block type Uniform (chunk.rs:127-134)
+        # block edits by chunk position: voxel index (z*1024 + y*32 + x) -> block type; kept while the chunk is unloaded and
+        # applied again when it is generated anew
+        self.edits: Dict[Pos, Dict[int, int]] = {}
         self._free: List[int] = list(range(self.capacity - 1, -1, -1))
         self.last_camera_chunk: Optional[Pos] = None
         self.generated_last_update: List[Pos] = []
@@ -178,6 +192,9 @@ class World:
         flags = self.device.generate(slots, np.array(new, dtype=np.int32).reshape(-1, 3))
         for p, f in zip(new, flags.tolist()):
             self.uniform_flags[p] = int(f)
+        edited = [p for p in new if p in self.edits]
+        if edited:
+            self._apply_edits([(p, i, t) for p in edited for i, t in self.edits[p].items()])
         touched = list(new)
         for p in new:  # the chunks next to a new one now have a neighbour there
             touched += [(p[0] + o[0], p[1] + o[1], p[2] + o[2]) for o in FACE_OFFSETS]
@@ -212,6 +229,81 @@ class World:
         for p in gone:  # their neighbours lose the reference to the slot (it will be reused)
             touched += [(p[0] + o[0], p[1] + o[1], p[2] + o[2]) for o in FACE_OFFSETS]
         self._push_neighbor_rows(touched)
+
+    # ---- block edits and picking (vx_world_batch_set_blocks, vx_world_raycast) ---------------------------------------------
+    def _apply_edits(self, edits: List[Tuple[Pos, int, int]]):
+        for p, _, _ in edits:
+            self.uniform_flags[p] = 0  # a Uniform chunk becomes Varied on its first edit
+        self.device.set_blocks(np.array([self.chunks[p] for p, _, _ in edits], dtype=np.int32),
+                               np.array([i for _, i, _ in edits], dtype=np.int32), np.array([t for _, _, t in edits], dtype=np.uint8))
+
+    def set_blocks(self, world_xyz, block_types) -> List[Pos]:
+        """Set the blocks at world voxel coordinates world_xyz (n, 3) to block_types (n,) or one type for all (0 = air .. 3);
+        when a voxel is listed twice the last entry wins.  Every chunk must be loaded (KeyError otherwise, before anything
+        changes).  The edits are recorded in `edits` and come back when a chunk is unloaded and generated again.  Nothing is
+        re-meshed: returns the positions whose meshes may change -- the edited chunks and the loaded neighbour across each
+        face on which an edited voxel lies (the mesher reads a neighbour only on the shared border plane) -- for
+        MeshCache.refresh."""
+        xyz = np.asarray(world_xyz, dtype=np.int64).reshape(-1, 3)
+        types = np.broadcast_to(np.asarray(block_types, dtype=np.int64).reshape(-1), (xyz.shape[0],))
+        if types.size and (types.min() < 0 or types.max() > 3):
+            raise ValueError("block types are 0..3")
+        cpos, local = xyz >> 5, xyz & 31
+        index = local[:, 2] * 1024 + local[:, 1] * 32 + local[:, 0]
+        edits = [(tuple(int(c) for c in cp), int(i), int(t)) for cp, i, t in zip(cpos, index, types)]
+        missing = sorted({p for p, _, _ in edits if p not in self.chunks})
+        if missing:
+            raise KeyError(f"set_blocks: chunks not loaded: {missing}")
+        if not edits:
+            return []
+        for p, i, t in edits:
+            self.edits.setdefault(p, {})[i] = t
+        self._apply_edits(edits)
+        dirty = set()
+        for (p, _, _), lp in zip(edits, local.tolist()):
+            dirty.add(p)
+            for a in range(3):
+                for border, face in ((31, 2 * a), (0, 2 * a + 1)):
+                    if lp[a] == border:
+                        o = FACE_OFFSETS[face]
+                        q = (p[0] + o[0], p[1] + o[1], p[2] + o[2])
+                        if q in self.chunks:
+                            dirty.add(q)
+        return sorted(dirty)
+
+    def start_slots(self, origins) -> np.ndarray:
+        """Slot of the chunk that holds each origin (world_to_chunk_pos), -1 where it is not loaded or not finite."""
+        o = np.asarray(origins, dtype=np.float32).reshape(-1, 3)
+        slots = np.full(o.shape[0], -1, dtype=np.int32)
+        with np.errstate(invalid="ignore", over="ignore"):
+            c = np.floor(o / np.float32(CHUNK_SIZE))
+        ok = np.isfinite(c).all(axis=1) & (np.abs(c) < 2.0 ** 30).all(axis=1)
+        if ok.any():
+            uniq, inv = np.unique(c[ok].astype(np.int64), axis=0, return_inverse=True)
+            found = np.array([self.chunks.get((int(u[0]), int(u[1]), int(u[2])), -1) for u in uniq], dtype=np.int32)
+            slots[ok] = found[inv.reshape(-1)]
+        return slots
+
+    def raycast(self, origins, dirs, max_t: float) -> Dict[str, np.ndarray]:
+        """vx_world_raycast (semantics in include/vx_b200.h) for rays starting in loaded chunks (others are RAY_INVALID).
+        Returns arrays per ray: status (RAY_HIT / _MISS / _LEFT_WORLD / _INVALID), chunk (the chunk position), local and
+        voxel (the hit voxel inside its chunk and in the world), face (FaceDir the ray entered through, -1 = the origin is
+        inside a solid voxel), block_type, t (o + t*d is the entry point) and distance (t * |d|; inf unless hit), plus
+        the raw VxRayHit records as `hits`."""
+        o = np.ascontiguousarray(origins, dtype=np.float32).reshape(-1, 3)
+        d = np.ascontiguousarray(dirs, dtype=np.float32).reshape(-1, 3)
+        hits = self.device.raycast(o, d, self.start_slots(o), float(max_t))
+        hit = hits["status"] == _lib.RAY_HIT
+        vox = hits["voxel"].astype(np.int32)
+        dist = np.where(hit, hits["t"].astype(np.float64) * np.linalg.norm(d.astype(np.float64), axis=1), np.inf)
+        return {"status": hits["status"].copy(), "chunk": vox >> 5, "local": vox & 31, "voxel": vox, "face": hits["face"].copy(),
+                "block_type": hits["block_type"].copy(), "t": hits["t"].copy(), "distance": dist, "hits": hits}
+
+    def pick(self, camera_position, view_proj, pixels, width: int, height: int, max_distance: float) -> Dict[str, np.ndarray]:
+        """What is under each pixel (n, 2) of a width x height frame: raycast along api.pixel_rays (unit directions, so
+        t is the distance from the camera), at most max_distance (<= 1e4) far."""
+        origins, dirs = api.pixel_rays(view_proj, camera_position, pixels, width, height)
+        return self.raycast(origins, dirs, max_distance)
 
     # ---- visibility world.rs:103-146 --------------------------------------------------------------------------------
     def get_visible_chunks(self, camera_position) -> List[Pos]:
@@ -261,6 +353,16 @@ class MeshCache:
         self.cached = {p for p in self.cached if w.contains_chunk(p)}  # main.rs:275
         self.meshed_last_frame = to_mesh
         return to_mesh
+
+    def refresh(self, positions: Iterable[Pos]) -> List[Pos]:
+        """Re-mesh, in one vx_world_batch_remesh call, those of `positions` (e.g. World.set_blocks' result) that have a
+        cache entry; the others are meshed when they first become visible.  Returns the re-meshed positions."""
+        w = self.world
+        todo = sorted({tuple(p) for p in positions} & self.cached)
+        todo = [p for p in todo if w.contains_chunk(p)]
+        if todo:
+            w.device.remesh(np.array([w.chunks[p] for p in todo], dtype=np.int32))
+        return todo
 
     def visible_mesh_slots(self, visible_chunks: Iterable[Pos]) -> np.ndarray:
         """Slots of the visible chunks that have a cache entry, in (x, y, z) order: the mesh_ids of vx_render_frame

@@ -232,6 +232,61 @@ VX_API int vx_world_batch_unload(VxContext *ctx, VxMeshBatch *b, const int32_t *
  * the same way.  Quads are appended to the stream; when it is full the live quads are compacted (copied, not
  * re-meshed). */
 VX_API int vx_world_batch_remesh(VxContext *ctx, VxMeshBatch *b, const int32_t *slots, int32_t n);
+/* Block edits: voxel voxel_index[i] (= z*1024 + y*32 + x inside the chunk) of slot slots[i] becomes block_types[i]
+ * (0..3), for n edits in list order -- when several edits name the same voxel, the last one wins.  A Uniform slot becomes
+ * Varied on its first edit: its 32 KiB are filled with its block type, its flag becomes 0, then the edits land (a chunk
+ * that ends up all air is still Varied; the mesher gives it no mesh, which draws like Uniform air).  Nothing is
+ * re-meshed: call vx_world_batch_remesh for the chunks whose meshes can change (the edited chunk, and the neighbour across
+ * each face on which an edited voxel lies).  Edit loaded slots only: an absent slot that is edited anyway becomes a
+ * Varied air chunk holding the edits, at whatever position its row last held, and stays so until the slot is generated
+ * again.  Stream ordered; synchronises before it returns. */
+VX_API int vx_world_batch_set_blocks(VxContext *ctx, VxMeshBatch *b, const int32_t *slots, const int32_t *voxel_index,
+                                     const uint8_t *block_types, int32_t n);
+
+/* ---- ray casting through a world batch (picking) -------------------------------------------------------------------
+ * One ray per thread, an Amanatides-Woo walk over the voxels the world batch holds; the exact semantics, which the CPU
+ * oracle (tests/ray_oracle.c: vxo_raycast) restates statement for statement, so that both give identical bits:
+ *   - ray i: origin o (f32 x 3, world units: voxel (x,y,z) occupies [x,x+1) x [y,y+1) x [z,z+1)), direction d (f32 x 3,
+ *     used as given, not normalised), start slot = the slot of the chunk that holds floor(o); the point at parameter t is
+ *     o + t*d.  max_t is one value per call.
+ *   - VX_RAY_INVALID: a non-finite component of o or d, d == (0,0,0), |o| >= 2^24 on some axis, max_t outside [0, 1e4]
+ *     (or NaN), a start slot outside [0, capacity) (-1 = "not loaded"), or a start slot whose position row is not the
+ *     floor division by 32 of the start voxel v = (floorf(o.x), floorf(o.y), floorf(o.z)).
+ *   - step on each axis: the sign of d (no step where the component is 0).  The parameter of the next voxel face on an
+ *     axis is computed in closed form whenever it is needed, tnext = ((float)plane - o) / d, with plane = v + 1 when
+ *     stepping up and plane = v when stepping down (v = the current voxel on that axis) -- never accumulated.
+ *   - the walk: if the current voxel is solid (type != 0) the ray hits it.  Else take the axis with the smallest tnext,
+ *     ties x before y before z; tnext > max_t -> VX_RAY_MISS; step the voxel on that axis; leaving the chunk through a
+ *     neighbour entry < 0 (VX_NBR_NONE: nothing loaded there) -> VX_RAY_LEFT_WORLD; else repeat in the new voxel.
+ *   - a Uniform chunk (flag != 0) has no voxel rows: a Uniform solid chunk is solid everywhere (type flag - 1; a ray that
+ *     enters it hits the entered voxel), a Uniform air chunk is walked without voxel loads.
+ *   - a hit reports status VX_RAY_HIT, the slot, the world voxel, its block type, t = the tnext of the step that entered
+ *     the voxel and face = the FaceDir (0..5 = +X,-X,+Y,-Y,+Z,-Z) of the hit voxel's face the ray crossed: a step towards
+ *     +x enters through -X, face 1.  An origin inside a solid voxel is a hit with t = 0 and face -1.  (A ray that starts
+ *     on a voxel face and steps down crosses that face at once, t = -0.0f.)
+ *   - every other status leaves slot = -1, voxel = (0,0,0), face = -1, t = 0, block_type = 0.
+ * The walk takes at most sum over the stepping axes of (floor(|d_axis| * max_t) + 3) steps (the planes within max_t, one
+ * for rounding, one for an origin on a face), so no ray runs unbounded; a -DVX_DEBUG_CHECKS build checks that bound inside
+ * the kernel, and vx_world_raycast then fails with VX_ERR_CUDA if a ray since the last call exceeded it. */
+enum { VX_RAY_HIT = 0, VX_RAY_MISS = 1, VX_RAY_LEFT_WORLD = 2, VX_RAY_INVALID = 3 };
+typedef struct {
+    int32_t status;   /* VX_RAY_* */
+    int32_t slot;     /* -1 unless hit */
+    int32_t voxel[3]; /* world voxel coordinates */
+    int32_t face;     /* FaceDir entered, -1 = origin inside a solid voxel */
+    float t;
+    uint8_t block_type, pad[3];
+} VxRayHit; /* 32 bytes */
+/* n rays from host arrays (origins / dirs n x 3 f32, start_slots n) into hits_out (n, host).  VX_ERR_INVALID for a batch
+ * that is not a world batch, a start slot outside [-1, capacity) or a missing array; a bad ray is reported through its
+ * status.  Synchronises before it returns. */
+VX_API int vx_world_raycast(VxContext *ctx, const VxMeshBatch *b, const float *origins, const float *dirs, const int32_t *start_slots,
+                            int32_t n, float max_t, VxRayHit *hits_out);
+/* The same kernel on arrays resident on the context's device; asynchronous on the context's stream.  Every bad ray,
+ * including a start slot out of range, is reported through its status (VX_ERR_INVALID only for a batch that is not a
+ * world batch or a missing array). */
+VX_API int vx_world_raycast_device(VxContext *ctx, const VxMeshBatch *b, const float *d_origins, const float *d_dirs,
+                                   const int32_t *d_start_slots, int32_t n, float max_t, VxRayHit *d_hits_out);
 
 /* ---- meshing ---------------------------------------------------------- */
 
