@@ -29,6 +29,9 @@ RAY_MISS = 1
 RAY_LEFT_WORLD = 2
 RAY_INVALID = 3
 
+MOVE_TOUCHED_UNLOADED = 1 << 6  # flag bits 0..5: the move along that FaceDir was blocked
+MOVE_INVALID = 1 << 7
+
 
 class VxError(RuntimeError):
     def __init__(self, code: int, msg: str):
@@ -148,6 +151,8 @@ PROTOTYPES = {
     "vx_world_batch_set_blocks": (C.c_int, [_P, _P, _P, _P, _P, _I]),
     "vx_world_raycast": (C.c_int, [_P, _P, _P, _P, _P, _I, C.c_float, _P]),
     "vx_world_raycast_device": (C.c_int, [_P, _P, _P, _P, _P, _I, C.c_float, _P]),
+    "vx_world_move_boxes": (C.c_int, [_P, _P, _P, _P, _P, _P, _I, _P]),
+    "vx_world_move_boxes_device": (C.c_int, [_P, _P, _P, _P, _P, _P, _I, _P]),
     "vx_render_mesh_tiny_quads": (C.c_int, [_P, _P, _I, _P, C.POINTER(VxFrameConfig), _P, _I, _P, _P]),
     "vx_render_mesh_with_up": (C.c_int, [_P, _P, _I, _P, C.POINTER(VxFrameConfig), _P, _P, _P]),
     "vx_render_frame_macrotile": (C.c_int, [_P, _P, _P, _I, _P, C.POINTER(VxFrameConfig), _P, _P, _P, C.POINTER(_I)]),

@@ -47,8 +47,8 @@ def sphere_capacity(view_distance: int) -> int:
 
 
 class _DeviceWorld:
-    """The vx_world_batch_* calls and vx_world_raycast; tests substitute a recorder for it to check the host logic without a
-    GPU."""
+    """The vx_world_batch_* calls, vx_world_raycast and vx_world_move_boxes; tests substitute a recorder for it to check the
+    host logic without a GPU."""
 
     def __init__(self, ctx: api.Context, capacity: int, terrain: VxTerrainParams):
         self.ctx = ctx
@@ -88,6 +88,13 @@ class _DeviceWorld:
         self.ctx.check(self.ctx.lib.vx_world_raycast(self.ctx.handle, self.batch.handle, api._p(origins), api._p(dirs), api._p(start_slots),
                                                      int(start_slots.size), float(max_t), api._p(hits)))
         return hits
+
+    def move_boxes(self, pos: np.ndarray, size: np.ndarray, delta: np.ndarray, slots: np.ndarray) -> np.ndarray:
+        """pos (n, 3) and slots (n,) are updated in place; returns the flags (n,)."""
+        flags = np.zeros(slots.size, dtype=np.uint32)
+        self.ctx.check(self.ctx.lib.vx_world_move_boxes(self.ctx.handle, self.batch.handle, api._p(pos), api._p(size), api._p(delta),
+                                                        api._p(slots), int(slots.size), api._p(flags)))
+        return flags
 
 
 class World:
@@ -304,6 +311,24 @@ class World:
         t is the distance from the camera), at most max_distance (<= 1e4) far."""
         origins, dirs = api.pixel_rays(view_proj, camera_position, pixels, width, height)
         return self.raycast(origins, dirs, max_distance)
+
+    # ---- collision (vx_world_move_boxes) -----------------------------------------------------------------------------
+    def move_boxes(self, pos, size, delta) -> Dict[str, np.ndarray]:
+        """Move boxes with min corner pos (n, 3) and extent size by delta through the loaded voxels, stopping at solid ones
+        and at unloaded space (vx_world_move_boxes; semantics in include/vx_b200.h: Y, then X, then Z).  size and delta
+        broadcast to (n, 3).  Gravity, jumping and stepping up are the caller's.  The caller's arrays are not modified.
+        Returns arrays per box: pos (the new min corner), slot (of the chunk holding floor(pos), -1 if not loaded), flags,
+        blocked ((n, 6) bool: the move along that FaceDir was cut short), on_ground (blocked moving -Y), touched_unloaded and
+        invalid (the box was left where it was)."""
+        p = np.array(pos, dtype=np.float32).reshape(-1, 3)
+        n = p.shape[0]
+        s = np.ascontiguousarray(np.broadcast_to(np.asarray(size, dtype=np.float32), (n, 3)))
+        d = np.ascontiguousarray(np.broadcast_to(np.asarray(delta, dtype=np.float32), (n, 3)))
+        slots = self.start_slots(p)
+        flags = self.device.move_boxes(p, s, d, slots)
+        blocked = ((flags[:, None] >> np.arange(6, dtype=np.uint32)) & 1).astype(bool)
+        return {"pos": p, "slot": slots, "flags": flags, "blocked": blocked, "on_ground": blocked[:, 3].copy(),
+                "touched_unloaded": (flags & _lib.MOVE_TOUCHED_UNLOADED) != 0, "invalid": (flags & _lib.MOVE_INVALID) != 0}
 
     # ---- visibility world.rs:103-146 --------------------------------------------------------------------------------
     def get_visible_chunks(self, camera_position) -> List[Pos]:

@@ -288,6 +288,56 @@ VX_API int vx_world_raycast(VxContext *ctx, const VxMeshBatch *b, const float *o
 VX_API int vx_world_raycast_device(VxContext *ctx, const VxMeshBatch *b, const float *d_origins, const float *d_dirs,
                                    const int32_t *d_start_slots, int32_t n, float max_t, VxRayHit *d_hits_out);
 
+/* ---- swept boxes through a world batch (collision) ------------------------------------------------------------------
+ * One box per thread, moved through the voxels the world batch holds and stopped at solid ones; the exact semantics, which
+ * the CPU oracle (tests/move_oracle.c: vxo_move_boxes) restates statement for statement, so that both give identical bits
+ * (every operation below is one correctly rounded f32 operation; fl(x) names its result):
+ *   - box i: min corner p = pos[i] and extent s = size[i] (f32 x 3, world units); it covers [p, max) on each axis with
+ *     max = fl(p + s), and voxel v on an axis when floor(p) <= v <= ceil(max) - 1.  It is displaced by delta[i] (f32 x 3).
+ *     Its slot is the slot of the chunk that holds floor(p), as for rays.
+ *   - VX_MOVE_INVALID (and nothing else) is reported, and pos[i] and the slot are left as they are, for: a non-finite
+ *     component of p, s or delta; |p| >= 2^20, s outside (0, 16], fl(p + s) <= p or |delta| > 16 on some axis; a slot
+ *     outside [0, capacity) (-1 = "not loaded"), or one whose position row is not floor(p) >> 5 (floor division by 32).
+ *     These bounds keep every voxel a move reads inside the 3 x 3 x 3 chunks around the slot's chunk; a -DVX_DEBUG_CHECKS
+ *     build checks that inside the kernel, and vx_world_move_boxes then fails with VX_ERR_CUDA if a box since the last
+ *     call left that neighbourhood.
+ *   - the chunk at offset (a, b, c) in {-1,0,1}^3 from the slot's chunk is reached through the neighbour rows: first the X
+ *     hop (a != 0: entry +X or -X), then Y, then Z.  A negative entry (VX_NBR_NONE) on that path means the chunk is not
+ *     loaded -- even if it is loaded and reachable along another path.  A voxel's type comes from the Uniform flag
+ *     (flag - 1) or the voxel bytes, as for rays.
+ *   - solid: a voxel whose type is not 0, or any voxel of a chunk that is not loaded (unloaded space is a wall, so nothing
+ *     falls out of the loaded world).
+ *   - the axes move one after the other, Y, then X, then Z (a falling box lands before it slides); each uses the position
+ *     the previous one left.  Axis a with d = delta[a] == 0 does nothing.  Else, with the cross-section voxels
+ *     floor(p_e) .. ceil(fl(p_e + s_e)) - 1 on each other axis e, and the candidate p' = fl(p_a + d):
+ *       d > 0: scan the layers L = ceil(fl(p_a + s_a)) .. ceil(fl(p' + s_a)) - 1 in ascending order.  At the first layer
+ *              with a solid voxel in the cross-section the move is blocked: p_a becomes the largest f32 m with
+ *              fl(m + s_a) <= (float)L.  The old p_a satisfies that and p' does not, so m is found by bisection over the
+ *              f32 values between them (at most 32 steps; stepping by ulps from fl(L - s_a) would take up to ~2^30 steps
+ *              when that guess is near 0, where the f32 are far denser than at L).  No block: p_a = p'.
+ *       d < 0: scan the layers L = floor(p_a) - 1 down to floor(p').  A block at L gives p_a = (float)(L + 1); no block:
+ *              p_a = p'.
+ *     A blocked move sets flag bit i of the FaceDir it was moving along (0..5 = +X,-X,+Y,-Y,+Z,-Z: a blocked +X move sets
+ *     bit 0, a blocked -Y move sets bit 3 = "on the ground"); VX_MOVE_TOUCHED_UNLOADED is set when a blocking layer holds
+ *     a voxel of a chunk that is not loaded.  The voxels a box already overlaps never block it (the scan starts beyond
+ *     them), so a box stuck inside a block can move out; a move never takes a box backwards (a blocked box stays at or
+ *     beyond where it was, short of p').  After the move, every voxel the box overlaps that it did not overlap before is
+ *     loaded and has type 0.
+ *   - output: pos[i] is updated in place, and the slot in place to the chunk holding the new floor(p) (reached by the same
+ *     hop rule; -1 if that chunk is not loaded), so the next call can take the arrays as they are.
+ * Flags per box: bits 0..5 as above, VX_MOVE_TOUCHED_UNLOADED, VX_MOVE_INVALID. */
+enum { VX_MOVE_TOUCHED_UNLOADED = 1 << 6, VX_MOVE_INVALID = 1 << 7 };
+/* n boxes from host arrays (pos_inout / size / delta n x 3 f32, slots_inout n), updated in place; flags_out (n, host).
+ * VX_ERR_INVALID for a batch that is not a world batch, a slot outside [-1, capacity) or a missing array; a bad box is
+ * reported through its flags.  Synchronises before it returns. */
+VX_API int vx_world_move_boxes(VxContext *ctx, const VxMeshBatch *b, float *pos_inout, const float *size, const float *delta,
+                               int32_t *slots_inout, int32_t n, uint32_t *flags_out);
+/* The same kernel on arrays resident on the context's device, updated in place, so that a physics loop can run tick after
+ * tick without the host; asynchronous on the context's stream.  Every bad box, including a slot out of range, is reported
+ * through its flags (VX_ERR_INVALID only for a batch that is not a world batch or a missing array). */
+VX_API int vx_world_move_boxes_device(VxContext *ctx, const VxMeshBatch *b, float *d_pos_inout, const float *d_size, const float *d_delta,
+                                      int32_t *d_slots_inout, int32_t n, uint32_t *d_flags_out);
+
 /* ---- meshing ---------------------------------------------------------- */
 
 /* BinaryGreedyMesher::mesh_world (binary_greedy.rs:62-78) / mesh_chunk_in_world (:83) /
