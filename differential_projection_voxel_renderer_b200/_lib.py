@@ -32,6 +32,10 @@ RAY_INVALID = 3
 MOVE_TOUCHED_UNLOADED = 1 << 6  # flag bits 0..5: the move along that FaceDir was blocked
 MOVE_INVALID = 1 << 7
 
+REGION_BOX = 0
+REGION_BALL = 1
+REGION_CHANGED = 1 << 6  # vx_world_batch_fill_regions change bits 0..5: a voxel on that FaceDir's border plane differs
+
 
 class VxError(RuntimeError):
     def __init__(self, code: int, msg: str):
@@ -89,6 +93,11 @@ class VxShardLayout(C.Structure):
 class VxRayHit(C.Structure):
     _fields_ = [("status", C.c_int32), ("slot", C.c_int32), ("voxel", C.c_int32 * 3), ("face", C.c_int32), ("t", C.c_float),
                 ("block_type", C.c_uint8), ("pad", C.c_uint8 * 3)]
+
+
+class VxRegionOp(C.Structure):
+    _fields_ = [("radius_sq", C.c_int64), ("shape", C.c_int32), ("a", C.c_int32 * 3), ("b", C.c_int32 * 3), ("block_type", C.c_uint8),
+                ("replace_mask", C.c_uint8), ("pad", C.c_uint8 * 2)]
 
 
 class VxFrameStats(C.Structure):
@@ -149,6 +158,8 @@ PROTOTYPES = {
     "vx_world_batch_unload": (C.c_int, [_P, _P, _P, _I]),
     "vx_world_batch_remesh": (C.c_int, [_P, _P, _P, _I]),
     "vx_world_batch_set_blocks": (C.c_int, [_P, _P, _P, _P, _P, _I]),
+    "vx_world_batch_fill_regions": (C.c_int, [_P, _P, _P, _I, _P, _I, _P]),
+    "vx_world_batch_read_voxels": (C.c_int, [_P, _P, _P, _I, _P, _P]),
     "vx_world_raycast": (C.c_int, [_P, _P, _P, _P, _P, _I, C.c_float, _P]),
     "vx_world_raycast_device": (C.c_int, [_P, _P, _P, _P, _P, _I, C.c_float, _P]),
     "vx_world_move_boxes": (C.c_int, [_P, _P, _P, _P, _P, _P, _I, _P]),

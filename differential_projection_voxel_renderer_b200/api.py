@@ -600,6 +600,12 @@ RAY_HIT_DTYPE = np.dtype([("status", "<i4"), ("slot", "<i4"), ("voxel", "<i4", (
                           ("block_type", "u1"), ("pad", "u1", (3,))])  # VxRayHit, 32 bytes
 assert RAY_HIT_DTYPE.itemsize == C.sizeof(_lib.VxRayHit)
 
+# ---- region edits (vx_world_batch_fill_regions) ---------------------------------------------------------------------
+
+REGION_OP_DTYPE = np.dtype([("radius_sq", "<i8"), ("shape", "<i4"), ("a", "<i4", (3,)), ("b", "<i4", (3,)), ("block_type", "u1"),
+                            ("replace_mask", "u1"), ("pad", "u1", (2,))])  # VxRegionOp, 40 bytes
+assert REGION_OP_DTYPE.itemsize == C.sizeof(_lib.VxRegionOp)
+
 
 def pixel_rays(view_proj, camera_position, pixels, width: int, height: int):
     """Rays from the camera through pixel centres, for vx_world_raycast: origin = camera_position, direction = the pixel

@@ -22,7 +22,9 @@
 //            Chunks with more quads than the pool holds re-run the merge and write directly.
 #include "vx_common.cuh"
 
+#include <cmath>
 #include <cstddef>
+#include <cstring>
 #include <memory>
 #include <unordered_set>
 #include <vector>
@@ -882,6 +884,104 @@ __global__ void scatter_blocks_kernel(uint8_t *voxels, const int32_t *slot, cons
     if (i < n) voxels[(size_t)slot[i] * VX_CHUNK_VOLUME + index[i]] = (uint8_t)type[i];
 }
 
+// vx_world_batch_fill_regions: a validated VxRegionOp with its world bounding box (a ball: centre +- isqrt(radius_sq)).
+struct RegionOp {
+    int32_t lo[3], hi[3], c[3], ball;
+    int64_t radius_sq;
+    uint32_t block_type, replace_mask;
+};
+
+// One CTA per listed slot.  Thread t owns the 16-byte words t + 256 k (k = 0..7): x = 16 (t & 1) .. +15, y = (t >> 1) & 31,
+// z = (t >> 6) + 4 k, so the whole chunk sits in registers, loaded once (built from the flag for a Uniform slot).  Every op
+// is applied in registers, skipping words outside its box clipped to the chunk; only words that differ at the end are
+// stored, or every word when a Uniform slot turns Varied.
+constexpr int FILL_THREADS = 256, FILL_WORDS = VX_CHUNK_VOLUME / 16 / FILL_THREADS;
+__global__ void __launch_bounds__(FILL_THREADS) fill_regions_kernel(uint8_t *voxels, uint8_t *flags, const int32_t *positions,
+                                                                    const RegionOp *__restrict__ ops, int32_t n_ops,
+                                                                    const int32_t *__restrict__ slots, uint8_t *changed) {
+    const int32_t s = slots[blockIdx.x];
+    const uint32_t flag = flags[s];
+    const int t = threadIdx.x, x0 = (t & 1) * 16, y = (t >> 1) & 31, z0 = t >> 6;
+    uint4 *row = reinterpret_cast<uint4 *>(voxels + (size_t)s * VX_CHUNK_VOLUME);
+    uint32_t cur[FILL_WORDS][4], orig[FILL_WORDS][4];
+    const uint32_t fill = (flag - 1) * 0x01010101u;
+#pragma unroll
+    for (int k = 0; k < FILL_WORDS; ++k) {
+        const uint4 w = flag ? make_uint4(fill, fill, fill, fill) : row[t + FILL_THREADS * k];
+        orig[k][0] = cur[k][0] = w.x;
+        orig[k][1] = cur[k][1] = w.y;
+        orig[k][2] = cur[k][2] = w.z;
+        orig[k][3] = cur[k][3] = w.w;
+    }
+    const int64_t base[3] = {(int64_t)positions[3 * s] * 32, (int64_t)positions[3 * s + 1] * 32, (int64_t)positions[3 * s + 2] * 32};
+    int wrote = 0; // some op changed a voxel of this thread's words at its time
+    for (int32_t i = 0; i < n_ops; ++i) {
+        const RegionOp op = ops[i];
+        int lo[3], hi[3];
+        bool empty = false;
+#pragma unroll
+        for (int e = 0; e < 3; ++e) { // the op's box clipped to the chunk, in local coordinates (the same in every thread)
+            lo[e] = (int)max((int64_t)op.lo[e] - base[e], (int64_t)0);
+            hi[e] = (int)min((int64_t)op.hi[e] - base[e], (int64_t)31);
+            empty |= lo[e] > hi[e];
+        }
+        if (empty || y < lo[1] || y > hi[1] || x0 + 15 < lo[0] || x0 > hi[0]) continue;
+        const int xa = max(lo[0], x0) - x0, xb = min(hi[0], x0 + 15) - x0; // 0..15
+        const uint32_t span = ((2u << xb) - 1u) & ~((1u << xa) - 1u);
+        const int64_t dy = base[1] + y - op.c[1];
+#pragma unroll
+        for (int k = 0; k < FILL_WORDS; ++k) {
+            const int z = z0 + 4 * k;
+            if (z < lo[2] || z > hi[2]) continue;
+            uint32_t in = span;
+            if (op.ball) {
+                const int64_t dz = base[2] + z - op.c[2];
+                const int64_t left = op.radius_sq - dy * dy - dz * dz;
+                const int64_t dx0 = base[0] + x0 - op.c[0];
+#pragma unroll
+                for (int j = 0; j < 16; ++j)
+                    if ((dx0 + j) * (dx0 + j) > left) in &= ~(1u << j);
+            }
+#pragma unroll
+            for (int j = 0; j < 16; ++j) {
+                const uint32_t sh = 8 * (j & 3), v = (cur[k][j >> 2] >> sh) & 0xFFu;
+                if (((in >> j) & 1u) && ((op.replace_mask >> v) & 1u) && v != op.block_type) {
+                    cur[k][j >> 2] = (cur[k][j >> 2] & ~(0xFFu << sh)) | (op.block_type << sh);
+                    wrote = 1;
+                }
+            }
+        }
+    }
+    // bits 0..5: a border voxel differs (FaceDir order), 6: some voxel differs
+    uint32_t bits = 0, differs = 0;
+#pragma unroll
+    for (int k = 0; k < FILL_WORDS; ++k) {
+        const uint32_t d0 = cur[k][0] ^ orig[k][0], d1 = cur[k][1] ^ orig[k][1], d2 = cur[k][2] ^ orig[k][2], d3 = cur[k][3] ^ orig[k][3];
+        if ((d0 | d1 | d2 | d3) == 0) continue;
+        const int z = z0 + 4 * k;
+        differs |= 1u << k;
+        bits |= 64u;
+        if (x0 == 16 && (d3 >> 24) != 0) bits |= 1u;
+        if (x0 == 0 && (d0 & 0xFFu) != 0) bits |= 2u;
+        if (y == 31) bits |= 4u;
+        if (y == 0) bits |= 8u;
+        if (z == 31) bits |= 16u;
+        if (z == 0) bits |= 32u;
+    }
+    __shared__ uint32_t s_bits;
+    if (t == 0) s_bits = 0;
+    __syncthreads();
+    if (bits) atomicOr(&s_bits, bits);
+    const int became_varied = __syncthreads_or(wrote) && flag != 0; // every thread has read the flag; s_bits is complete
+#pragma unroll
+    for (int k = 0; k < FILL_WORDS; ++k)
+        if (became_varied || ((differs >> k) & 1u)) row[t + FILL_THREADS * k] = make_uint4(cur[k][0], cur[k][1], cur[k][2], cur[k][3]);
+    if (t == 0) {
+        if (became_varied) flags[s] = 0;
+        changed[blockIdx.x] = (uint8_t)(s_bits | (became_varied ? 64u : 0u));
+    }
+}
+
 } // namespace
 
 extern "C" {
@@ -1388,6 +1488,81 @@ int vx_world_batch_set_blocks(VxContext *ctx, VxMeshBatch *b, const int32_t *slo
                                                                                   (int32_t)k);
     VX_CHECK_LAUNCH(ctx);
     VX_CUDA(ctx, cudaStreamSynchronize(ctx->stream)); // `staged` goes out of scope
+    return VX_OK;
+}
+
+int vx_world_batch_fill_regions(VxContext *ctx, VxMeshBatch *b, const VxRegionOp *ops, int32_t n_ops, const int32_t *slots, int32_t n_slots,
+                                uint8_t *changed_out) {
+    int rc = world_check_slots(ctx, b, slots, n_slots, "vx_world_batch_fill_regions: bad argument");
+    if (rc != VX_OK) return rc;
+    if (n_ops < 0 || (n_ops > 0 && !ops) || (n_slots > 0 && !changed_out)) return vx_fail(ctx, VX_ERR_INVALID, "vx_world_batch_fill_regions: bad argument");
+    std::vector<uint8_t> listed((size_t)b->n_chunks, 0);
+    for (int32_t i = 0; i < n_slots; ++i)
+        if (listed[slots[i]]++) return vx_fail(ctx, VX_ERR_INVALID, "vx_world_batch_fill_regions: slot listed twice");
+    constexpr int32_t COORD = 1 << 29;
+    constexpr int64_t RADIUS_SQ = (int64_t)1 << 56;
+    std::vector<RegionOp> dev((size_t)n_ops);
+    for (int32_t i = 0; i < n_ops; ++i) {
+        const VxRegionOp &o = ops[i];
+        const bool ball = o.shape == VX_REGION_BALL;
+        if ((o.shape != VX_REGION_BOX && !ball) || o.block_type > 3 || o.replace_mask > 15)
+            return vx_fail(ctx, VX_ERR_INVALID, "vx_world_batch_fill_regions: bad shape, block type or replace mask");
+        if (ball && (o.radius_sq < 0 || o.radius_sq > RADIUS_SQ))
+            return vx_fail(ctx, VX_ERR_INVALID, "vx_world_batch_fill_regions: radius_sq out of range");
+        int32_t r = 0;
+        if (ball) { // floor(sqrt(radius_sq)), exact
+            int64_t q = (int64_t)std::sqrt((double)o.radius_sq);
+            while (q * q > o.radius_sq) --q;
+            while ((q + 1) * (q + 1) <= o.radius_sq) ++q;
+            r = (int32_t)q;
+        }
+        RegionOp &d = dev[(size_t)i];
+        for (int e = 0; e < 3; ++e) {
+            if (o.a[e] < -COORD || o.a[e] > COORD || (!ball && (o.b[e] < -COORD || o.b[e] > COORD)))
+                return vx_fail(ctx, VX_ERR_INVALID, "vx_world_batch_fill_regions: coordinate out of range");
+            d.lo[e] = ball ? o.a[e] - r : o.a[e];
+            d.hi[e] = ball ? o.a[e] + r : o.b[e];
+            d.c[e] = o.a[e];
+        }
+        d.ball = ball;
+        d.radius_sq = o.radius_sq;
+        d.block_type = o.block_type;
+        d.replace_mask = o.replace_mask;
+    }
+    if (n_slots == 0) return VX_OK;
+    if (n_ops == 0) {
+        memset(changed_out, 0, (size_t)n_slots);
+        return VX_OK;
+    }
+    VX_CUDA(ctx, cudaSetDevice(ctx->device));
+    // staged: ops, then slots, then the change bytes the kernel writes
+    const size_t ops_bytes = sizeof(RegionOp) * dev.size(), slot_bytes = sizeof(int32_t) * (size_t)n_slots;
+    VX_CUDA(ctx, ctx->tmp_a.reserve(ops_bytes + slot_bytes + (size_t)n_slots));
+    uint8_t *d = ctx->tmp_a.as<uint8_t>();
+    VX_CUDA(ctx, cudaMemcpyAsync(d, dev.data(), ops_bytes, cudaMemcpyHostToDevice, ctx->stream));
+    VX_CUDA(ctx, cudaMemcpyAsync(d + ops_bytes, slots, slot_bytes, cudaMemcpyHostToDevice, ctx->stream));
+    fill_regions_kernel<<<(unsigned)n_slots, FILL_THREADS, 0, ctx->stream>>>(
+        b->world_voxels.as<uint8_t>(), b->world_flags.as<uint8_t>(), b->positions.as<int32_t>(), reinterpret_cast<const RegionOp *>(d), n_ops,
+        reinterpret_cast<const int32_t *>(d + ops_bytes), d + ops_bytes + slot_bytes);
+    VX_CHECK_LAUNCH(ctx);
+    VX_CUDA(ctx, cudaMemcpyAsync(changed_out, d + ops_bytes + slot_bytes, (size_t)n_slots, cudaMemcpyDeviceToHost, ctx->stream));
+    VX_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+    return VX_OK;
+}
+
+int vx_world_batch_read_voxels(VxContext *ctx, const VxMeshBatch *b, const int32_t *slots, int32_t n, uint8_t *voxels_out, uint8_t *flags_out) {
+    int rc = world_check_slots(ctx, b, slots, n, "vx_world_batch_read_voxels: bad argument");
+    if (rc != VX_OK || n == 0) return rc;
+    if (!flags_out) return vx_fail(ctx, VX_ERR_INVALID, "vx_world_batch_read_voxels: bad argument");
+    VX_CUDA(ctx, cudaSetDevice(ctx->device));
+    for (int32_t i = 0; i < n; ++i) {
+        const size_t s = (size_t)slots[i];
+        if (voxels_out)
+            VX_CUDA(ctx, cudaMemcpyAsync(voxels_out + (size_t)i * VX_CHUNK_VOLUME, b->world_voxels.as<uint8_t>() + s * VX_CHUNK_VOLUME, VX_CHUNK_VOLUME,
+                                         cudaMemcpyDeviceToHost, ctx->stream));
+        VX_CUDA(ctx, cudaMemcpyAsync(flags_out + i, b->world_flags.as<uint8_t>() + s, 1, cudaMemcpyDeviceToHost, ctx->stream));
+    }
+    VX_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
     return VX_OK;
 }
 

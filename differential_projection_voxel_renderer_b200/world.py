@@ -9,6 +9,7 @@ Nothing here generates, meshes or draws on the CPU.
 from __future__ import annotations
 
 import ctypes as C
+import math
 from typing import Dict, Iterable, List, Optional, Tuple
 
 import numpy as np
@@ -46,9 +47,38 @@ def sphere_capacity(view_distance: int) -> int:
     return int(((x * x + y * y + z * z) <= r * r).sum())
 
 
+REGION_COORD, REGION_RADIUS_SQ = 1 << 29, 1 << 56  # the bounds of vx_world_batch_fill_regions
+
+
+def _region_op(shape: int, a, b, radius_sq: int, block_type: int, replace) -> np.ndarray:
+    """A checked VxRegionOp record (api.REGION_OP_DTYPE); ValueError for what vx_world_batch_fill_regions would refuse."""
+    types = range(4) if replace is None else [int(t) for t in replace]
+    if not 0 <= int(block_type) <= 3 or any(not 0 <= t <= 3 for t in types):
+        raise ValueError("block types are 0..3")
+    a, b = np.asarray(a, dtype=np.int64).reshape(3), np.asarray(b, dtype=np.int64).reshape(3)
+    if (np.abs(a) > REGION_COORD).any() or (np.abs(b) > REGION_COORD).any() or int(radius_sq) > REGION_RADIUS_SQ:
+        raise ValueError("region coordinates are limited to [-2^29, 2^29] and radius_sq to 2^56")
+    op = np.zeros((), dtype=api.REGION_OP_DTYPE)
+    op["shape"], op["a"], op["b"], op["radius_sq"] = shape, a, b, int(radius_sq)
+    op["block_type"], op["replace_mask"] = int(block_type), sum(1 << t for t in set(types))
+    return op
+
+
+def region_contains(op: np.ndarray, voxels: np.ndarray) -> np.ndarray:
+    """Which world voxels (n, 3) lie inside the region of a VxRegionOp record (include/vx_b200.h)."""
+    v = np.asarray(voxels, dtype=np.int64).reshape(-1, 3)
+    a = op["a"].astype(np.int64)
+    if int(op["shape"]) == _lib.REGION_BOX:
+        return ((v >= a) & (v <= op["b"].astype(np.int64))).all(axis=1)
+    d = v - a
+    r = math.isqrt(int(op["radius_sq"]))
+    near = (np.abs(d) <= r).all(axis=1)
+    return near & ((np.where(near[:, None], d, 0) ** 2).sum(axis=1) <= int(op["radius_sq"]))
+
+
 class _DeviceWorld:
-    """The vx_world_batch_* calls, vx_world_raycast and vx_world_move_boxes; tests substitute a recorder for it to check the
-    host logic without a GPU."""
+    """The vx_world_batch_* calls (block and region edits included), vx_world_raycast and vx_world_move_boxes; tests
+    substitute a recorder for it to check the host logic without a GPU."""
 
     def __init__(self, ctx: api.Context, capacity: int, terrain: VxTerrainParams):
         self.ctx = ctx
@@ -83,6 +113,21 @@ class _DeviceWorld:
         self.ctx.check(self.ctx.lib.vx_world_batch_set_blocks(self.ctx.handle, self.batch.handle, api._p(slots), api._p(voxel_index),
                                                               api._p(block_types), int(slots.size)))
 
+    def fill_regions(self, ops: np.ndarray, slots: np.ndarray) -> np.ndarray:
+        """ops: api.REGION_OP_DTYPE records; returns the change bits per slot."""
+        changed = np.zeros(slots.size, dtype=np.uint8)
+        self.ctx.check(self.ctx.lib.vx_world_batch_fill_regions(self.ctx.handle, self.batch.handle, api._p(ops), int(ops.size), api._p(slots),
+                                                                int(slots.size), api._p(changed)))
+        return changed
+
+    def read_voxels(self, slots: np.ndarray) -> Tuple[np.ndarray, np.ndarray]:
+        """The raw voxel rows (n, 32768) and Uniform flags (n,) of the slots."""
+        voxels = np.zeros((slots.size, CHUNK_SIZE ** 3), dtype=np.uint8)
+        flags = np.zeros(slots.size, dtype=np.uint8)
+        self.ctx.check(self.ctx.lib.vx_world_batch_read_voxels(self.ctx.handle, self.batch.handle, api._p(slots), int(slots.size),
+                                                               api._p(voxels), api._p(flags)))
+        return voxels, flags
+
     def raycast(self, origins: np.ndarray, dirs: np.ndarray, start_slots: np.ndarray, max_t: float) -> np.ndarray:
         hits = np.zeros(start_slots.size, dtype=api.RAY_HIT_DTYPE)
         self.ctx.check(self.ctx.lib.vx_world_raycast(self.ctx.handle, self.batch.handle, api._p(origins), api._p(dirs), api._p(start_slots),
@@ -111,6 +156,10 @@ class World:
         # block edits by chunk position: voxel index (z*1024 + y*32 + x) -> block type; kept while the chunk is unloaded and
         # applied again when it is generated anew
         self.edits: Dict[Pos, Dict[int, int]] = {}
+        # region fills (fill_box / fill_ball; api.REGION_OP_DTYPE records) in issue order, and per chunk position the indices
+        # of the fills that changed it: replayed, before `edits`, when the chunk is generated anew
+        self.fills: List[np.ndarray] = []
+        self._fills_at: Dict[Pos, List[int]] = {}
         self._free: List[int] = list(range(self.capacity - 1, -1, -1))
         self.last_camera_chunk: Optional[Pos] = None
         self.generated_last_update: List[Pos] = []
@@ -199,6 +248,13 @@ class World:
         flags = self.device.generate(slots, np.array(new, dtype=np.int32).reshape(-1, 3))
         for p, f in zip(new, flags.tolist()):
             self.uniform_flags[p] = int(f)
+        refill = [p for p in new if p in self._fills_at]
+        if refill:
+            ops = np.stack([self.fills[i] for i in sorted({i for p in refill for i in self._fills_at[p]})])
+            changed = self.device.fill_regions(ops, np.array([self.chunks[p] for p in refill], dtype=np.int32))
+            for p, c in zip(refill, changed.tolist()):
+                if c & _lib.REGION_CHANGED:
+                    self.uniform_flags[p] = 0
         edited = [p for p in new if p in self.edits]
         if edited:
             self._apply_edits([(p, i, t) for p in edited for i, t in self.edits[p].items()])
@@ -277,6 +333,80 @@ class World:
                         if q in self.chunks:
                             dirty.add(q)
         return sorted(dirty)
+
+    # ---- region edits (vx_world_batch_fill_regions) ----------------------------------------------------------------
+    def fill_box(self, lo, hi, block_type: int, replace: Optional[Iterable[int]] = None) -> List[Pos]:
+        """Set the voxels of the box lo..hi (world voxel coordinates, both corners inclusive) whose type is in `replace` (block
+        types; None = all four) to block_type.  See fill_ball for what is returned and kept."""
+        op = _region_op(_lib.REGION_BOX, lo, hi, 0, block_type, replace)
+        lo, hi = op["a"].astype(np.int64), op["b"].astype(np.int64)
+        if (lo > hi).any():
+            return []
+        return self._fill(op, self._chunks_between(lo >> 5, hi >> 5))
+
+    def fill_ball(self, centre, radius_sq: int, block_type: int, replace: Optional[Iterable[int]] = None) -> List[Pos]:
+        """Set the voxels v with |v - centre|^2 <= radius_sq (world voxel coordinates, integers) whose type is in `replace` (block
+        types; None = all four) to block_type: carve an explosion with fill_ball(c, r2, 0, replace=(1, 2, 3)).  Exact semantics
+        in include/vx_b200.h (vx_world_batch_fill_regions).  Every chunk that holds a voxel of the ball must be loaded
+        (KeyError otherwise, before anything changes); a ball with radius_sq < 0 is empty and returns [] without a device
+        call.  The fill is recorded and comes back when a chunk is unloaded and generated again (fills first, in issue order,
+        then `edits`, into which every fill is folded).  Nothing is re-meshed: returns the positions whose meshes may change --
+        the chunks whose voxels or Uniform flag changed and the loaded neighbour across each face on which a voxel changed --
+        for MeshCache.refresh."""
+        op = _region_op(_lib.REGION_BALL, centre, (0, 0, 0), radius_sq, block_type, replace)
+        if int(op["radius_sq"]) < 0:
+            return []
+        a, r = op["a"].astype(np.int64), math.isqrt(int(op["radius_sq"]))
+        box = self._chunks_between((a - r) >> 5, (a + r) >> 5)
+        near = np.clip(a, box * CHUNK_SIZE, box * CHUNK_SIZE + CHUNK_SIZE - 1) - a  # the point of each chunk nearest the centre
+        return self._fill(op, box[(near * near).sum(axis=1) <= int(op["radius_sq"])])
+
+    def _chunks_between(self, c0: np.ndarray, c1: np.ndarray) -> np.ndarray:
+        """Chunk positions c0 .. c1 (inclusive) as (n, 3) int64 in (x, y, z) order; KeyError when the range reaches beyond the
+        loaded chunks on some axis (a region's chunks span its whole range on each axis, so one of them is not loaded)."""
+        loaded = np.array(list(self.chunks), dtype=np.int64).reshape(-1, 3)
+        if loaded.size == 0 or (c0 < loaded.min(axis=0)).any() or (c1 > loaded.max(axis=0)).any():
+            raise KeyError(f"fill: chunks {tuple(c0.tolist())} .. {tuple(c1.tolist())} reach beyond the loaded world")
+        axes = [np.arange(int(u), int(v) + 1) for u, v in zip(c0, c1)]
+        return np.stack(np.meshgrid(*axes, indexing="ij"), axis=-1).reshape(-1, 3)
+
+    def _fill(self, op: np.ndarray, touched: np.ndarray) -> List[Pos]:
+        touched = [tuple(int(c) for c in p) for p in touched]
+        missing = [p for p in touched if p not in self.chunks]
+        if missing:
+            raise KeyError(f"fill: chunks not loaded: {missing[:16]}{' ...' if len(missing) > 16 else ''}")
+        changed = self.device.fill_regions(op.reshape(1), np.array([self.chunks[p] for p in touched], dtype=np.int32))
+        k = len(self.fills)
+        self.fills.append(op)
+        dirty = set()
+        for p, c in zip(touched, changed.tolist()):
+            if not c & _lib.REGION_CHANGED:
+                continue  # unchanged: replaying the fill there would change nothing but voxels that `edits` sets anyway
+            self._fills_at.setdefault(p, []).append(k)
+            self.uniform_flags[p] = 0
+            dirty.add(p)
+            for f, o in enumerate(FACE_OFFSETS):
+                q = (p[0] + o[0], p[1] + o[1], p[2] + o[2])
+                if (c >> f) & 1 and q in self.chunks:
+                    dirty.add(q)
+            e = self.edits.get(p)
+            if e:  # fold: an edited voxel inside the shape whose type is in the mask now holds block_type
+                idx = np.fromiter(e.keys(), dtype=np.int64, count=len(e))
+                types = np.fromiter(e.values(), dtype=np.int64, count=len(e))
+                v = np.stack([idx & 31, (idx >> 5) & 31, idx >> 10], axis=1) + np.array(p, dtype=np.int64) * CHUNK_SIZE
+                hit = region_contains(op, v) & (((int(op["replace_mask"]) >> types) & 1) == 1)
+                for i in idx[hit].tolist():
+                    e[i] = int(op["block_type"])
+        return sorted(dirty)
+
+    def chunk_voxels(self, pos) -> Tuple[int, np.ndarray]:
+        """(Uniform flag, voxels) of a loaded chunk read back from the device (vx_world_batch_read_voxels): flag 0 Varied, else
+        1 + block type; voxels (32, 32, 32) uint8 indexed [z, y, x] -- a Uniform chunk's are all its type."""
+        voxels, flags = self.device.read_voxels(np.array([self.chunks[tuple(pos)]], dtype=np.int32))
+        v = voxels[0].reshape(CHUNK_SIZE, CHUNK_SIZE, CHUNK_SIZE)
+        if flags[0]:
+            v[:] = flags[0] - 1
+        return int(flags[0]), v
 
     def start_slots(self, origins) -> np.ndarray:
         """Slot of the chunk that holds each origin (world_to_chunk_pos), -1 where it is not loaded or not finite."""

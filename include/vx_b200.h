@@ -243,6 +243,49 @@ VX_API int vx_world_batch_remesh(VxContext *ctx, VxMeshBatch *b, const int32_t *
 VX_API int vx_world_batch_set_blocks(VxContext *ctx, VxMeshBatch *b, const int32_t *slots, const int32_t *voxel_index,
                                      const uint8_t *block_types, int32_t n);
 
+/* ---- region edits: fill or carve boxes and balls of a world batch ----------------------------------------------------
+ * The exact semantics, which the CPU oracle (tests/region_oracle.c: vxo_fill_regions) restates statement for statement, all
+ * in integer arithmetic:
+ *   - each listed slot applies ops 0 .. n_ops-1 in order to its own voxels.  Voxel (x, y, z) of a slot (local 0..31, index
+ *     z*1024 + y*32 + x) is world voxel v = position * 32 + local.  A voxel inside the op's shape whose current type t has
+ *     bit t set in replace_mask becomes block_type; every other voxel is left as it is (voxels outside every shape are never
+ *     written).
+ *   - VX_REGION_BOX: v is inside iff a[e] <= v[e] <= b[e] on every axis e (a box with a[e] > b[e] holds nothing).
+ *     VX_REGION_BALL: v is inside iff |v[e] - a[e]| <= r on every axis, with r = floor(sqrt(radius_sq)), and
+ *     sum over e of (v[e] - a[e])^2 <= radius_sq (the first condition follows from the second; testing it first keeps
+ *     every product inside int64).  b is ignored.
+ *   - VX_ERR_INVALID, before anything changes, for: a batch that is not a world batch; a slot outside [0, capacity) or
+ *     listed twice; a shape other than the two; block_type > 3; replace_mask > 15; a coordinate of a (or of b for a box)
+ *     outside [-2^29, 2^29]; radius_sq outside [0, 2^56] for a ball.  Within these bounds |v[e] - a[e]| <= 2^28 for every
+ *     voxel tested, so the sum of squares stays below 2^58.
+ *   - Uniform slots: a Uniform slot becomes Varied at the first op that changes one of its voxels (a voxel whose type is
+ *     in the mask and differs from block_type): its rows are filled with its type, its flag becomes 0, then the op lands.
+ *     It stays Varied even if later ops restore every voxel.  A Uniform slot none of whose voxels any op changes keeps its
+ *     flag, and its rows are not written.  (vx_world_batch_set_blocks differs: it makes a slot Varied on any edit.)
+ *   - changed_out[i] (host, n_slots bytes) for slots[i]: bit 6 is set when the slot's voxels or its Uniform flag differ
+ *     from before the call; bit f (0..5, FaceDir order +X,-X,+Y,-Y,+Z,-Z) is set when a voxel on that border plane
+ *     (+X: x = 31, -X: x = 0, +Y: y = 31, ...) differs from before the call.  A slot whose voxels all come back to their
+ *     old types has no face bit, and bit 6 only if it turned Varied.
+ * Nothing is re-meshed: call vx_world_batch_remesh for the slots with bit 6 and the neighbour across each face bit (the
+ * mesher reads a neighbour only on the shared border plane).  Fill loaded slots only, as for vx_world_batch_set_blocks.
+ * Stream ordered; synchronises before it returns. */
+enum { VX_REGION_BOX = 0, VX_REGION_BALL = 1 };
+typedef struct {
+    int64_t radius_sq;     /* ball: voxel v is inside iff |v - a|^2 <= radius_sq */
+    int32_t shape;         /* VX_REGION_* */
+    int32_t a[3], b[3];    /* box: inclusive min / max world voxel; ball: a = centre voxel, b ignored */
+    uint8_t block_type;    /* 0..3 */
+    uint8_t replace_mask;  /* bit t set: voxels of type t are overwritten (0xF = all) */
+    uint8_t pad[2];
+} VxRegionOp; /* 40 bytes */
+VX_API int vx_world_batch_fill_regions(VxContext *ctx, VxMeshBatch *b, const VxRegionOp *ops, int32_t n_ops,
+                                       const int32_t *slots, int32_t n_slots, uint8_t *changed_out);
+/* The voxel rows (voxels_out: n x 32768 bytes, may be NULL) and Uniform flags (flags_out: n bytes, 0 Varied, else 1 +
+ * block type) of the listed slots, copied as they are: the rows of a Uniform slot are not its voxels (its flag is).
+ * A plain synchronous copy. */
+VX_API int vx_world_batch_read_voxels(VxContext *ctx, const VxMeshBatch *b, const int32_t *slots, int32_t n, uint8_t *voxels_out,
+                                      uint8_t *flags_out);
+
 /* ---- ray casting through a world batch (picking) -------------------------------------------------------------------
  * One ray per thread, an Amanatides-Woo walk over the voxels the world batch holds; the exact semantics, which the CPU
  * oracle (tests/ray_oracle.c: vxo_raycast) restates statement for statement, so that both give identical bits:
