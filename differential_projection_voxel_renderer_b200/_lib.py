@@ -36,6 +36,8 @@ REGION_BOX = 0
 REGION_BALL = 1
 REGION_CHANGED = 1 << 6  # vx_world_batch_fill_regions change bits 0..5: a voxel on that FaceDir's border plane differs
 
+PASTE_SKIP = 0xFF  # vx_world_batch_paste: a template byte that leaves its voxel alone; vx_world_batch_copy_region: not loaded
+
 
 class VxError(RuntimeError):
     def __init__(self, code: int, msg: str):
@@ -100,6 +102,11 @@ class VxRegionOp(C.Structure):
                 ("replace_mask", C.c_uint8), ("pad", C.c_uint8 * 2)]
 
 
+class VxPasteOp(C.Structure):
+    _fields_ = [("offset", C.c_int64), ("origin", C.c_int32 * 3), ("dims", C.c_int32 * 3), ("replace_mask", C.c_uint8),
+                ("pad", C.c_uint8 * 7)]
+
+
 class VxFrameStats(C.Structure):
     _fields_ = [("n_input", C.c_int32), ("n_survivors", C.c_int32), ("n_quads", C.c_int32),
                 ("n_triangles", C.c_int32), ("n_bin_entries", C.c_int32), ("n_kernel_launches", C.c_int32),
@@ -160,6 +167,8 @@ PROTOTYPES = {
     "vx_world_batch_set_blocks": (C.c_int, [_P, _P, _P, _P, _P, _I]),
     "vx_world_batch_fill_regions": (C.c_int, [_P, _P, _P, _I, _P, _I, _P]),
     "vx_world_batch_read_voxels": (C.c_int, [_P, _P, _P, _I, _P, _P]),
+    "vx_world_batch_copy_region": (C.c_int, [_P, _P, _P, _P, _P, _P]),
+    "vx_world_batch_paste": (C.c_int, [_P, _P, _P, _I, _P, C.c_int64, _P, _I, _P]),
     "vx_world_raycast": (C.c_int, [_P, _P, _P, _P, _P, _I, C.c_float, _P]),
     "vx_world_raycast_device": (C.c_int, [_P, _P, _P, _P, _P, _I, C.c_float, _P]),
     "vx_world_move_boxes": (C.c_int, [_P, _P, _P, _P, _P, _P, _I, _P]),

@@ -606,6 +606,13 @@ REGION_OP_DTYPE = np.dtype([("radius_sq", "<i8"), ("shape", "<i4"), ("a", "<i4",
                             ("replace_mask", "u1"), ("pad", "u1", (2,))])  # VxRegionOp, 40 bytes
 assert REGION_OP_DTYPE.itemsize == C.sizeof(_lib.VxRegionOp)
 
+# ---- copy and paste (vx_world_batch_copy_region, vx_world_batch_paste) ------------------------------------------------
+
+PASTE_SKIP = _lib.PASTE_SKIP
+PASTE_OP_DTYPE = np.dtype([("offset", "<i8"), ("origin", "<i4", (3,)), ("dims", "<i4", (3,)), ("replace_mask", "u1"),
+                           ("pad", "u1", (7,))])  # VxPasteOp, 40 bytes
+assert PASTE_OP_DTYPE.itemsize == C.sizeof(_lib.VxPasteOp)
+
 
 def pixel_rays(view_proj, camera_position, pixels, width: int, height: int):
     """Rays from the camera through pixel centres, for vx_world_raycast: origin = camera_position, direction = the pixel

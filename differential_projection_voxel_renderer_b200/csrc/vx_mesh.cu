@@ -891,19 +891,12 @@ struct RegionOp {
     uint32_t block_type, replace_mask;
 };
 
-// One CTA per listed slot.  Thread t owns the 16-byte words t + 256 k (k = 0..7): x = 16 (t & 1) .. +15, y = (t >> 1) & 31,
-// z = (t >> 6) + 4 k, so the whole chunk sits in registers, loaded once (built from the flag for a Uniform slot).  Every op
-// is applied in registers, skipping words outside its box clipped to the chunk; only words that differ at the end are
-// stored, or every word when a Uniform slot turns Varied.
+// A chunk held in registers by one CTA of FILL_THREADS (fill_regions_kernel, paste_kernel).  Thread t owns the 16-byte
+// words t + 256 k (k = 0..7): x = 16 (t & 1) .. +15, y = (t >> 1) & 31, z = (t >> 6) + 4 k, so the whole chunk is loaded
+// once (built from the flag for a Uniform slot); ops edit `cur`, `orig` keeps the words as loaded.
 constexpr int FILL_THREADS = 256, FILL_WORDS = VX_CHUNK_VOLUME / 16 / FILL_THREADS;
-__global__ void __launch_bounds__(FILL_THREADS) fill_regions_kernel(uint8_t *voxels, uint8_t *flags, const int32_t *positions,
-                                                                    const RegionOp *__restrict__ ops, int32_t n_ops,
-                                                                    const int32_t *__restrict__ slots, uint8_t *changed) {
-    const int32_t s = slots[blockIdx.x];
-    const uint32_t flag = flags[s];
-    const int t = threadIdx.x, x0 = (t & 1) * 16, y = (t >> 1) & 31, z0 = t >> 6;
-    uint4 *row = reinterpret_cast<uint4 *>(voxels + (size_t)s * VX_CHUNK_VOLUME);
-    uint32_t cur[FILL_WORDS][4], orig[FILL_WORDS][4];
+__device__ __forceinline__ void load_chunk_words(const uint4 *row, uint32_t flag, int t, uint32_t (&cur)[FILL_WORDS][4],
+                                                 uint32_t (&orig)[FILL_WORDS][4]) {
     const uint32_t fill = (flag - 1) * 0x01010101u;
 #pragma unroll
     for (int k = 0; k < FILL_WORDS; ++k) {
@@ -913,6 +906,55 @@ __global__ void __launch_bounds__(FILL_THREADS) fill_regions_kernel(uint8_t *vox
         orig[k][2] = cur[k][2] = w.z;
         orig[k][3] = cur[k][3] = w.w;
     }
+}
+
+// The end of a chunk edit: the change byte (bits 0..5: a border voxel differs, FaceDir order; 6: some voxel differs or a
+// Uniform slot turned Varied) and the store-back of the words that differ, or of every word when a Uniform slot turns
+// Varied.  `wrote`: some op changed a voxel of this thread's words at its time.
+__device__ __forceinline__ void store_chunk_words(uint4 *row, uint8_t *flags, int32_t s, uint32_t flag, int t, int wrote,
+                                                  const uint32_t (&cur)[FILL_WORDS][4], const uint32_t (&orig)[FILL_WORDS][4],
+                                                  uint8_t *changed) {
+    const int x0 = (t & 1) * 16, y = (t >> 1) & 31, z0 = t >> 6;
+    uint32_t bits = 0, differs = 0;
+#pragma unroll
+    for (int k = 0; k < FILL_WORDS; ++k) {
+        const uint32_t d0 = cur[k][0] ^ orig[k][0], d1 = cur[k][1] ^ orig[k][1], d2 = cur[k][2] ^ orig[k][2], d3 = cur[k][3] ^ orig[k][3];
+        if ((d0 | d1 | d2 | d3) == 0) continue;
+        const int z = z0 + 4 * k;
+        differs |= 1u << k;
+        bits |= 64u;
+        if (x0 == 16 && (d3 >> 24) != 0) bits |= 1u;
+        if (x0 == 0 && (d0 & 0xFFu) != 0) bits |= 2u;
+        if (y == 31) bits |= 4u;
+        if (y == 0) bits |= 8u;
+        if (z == 31) bits |= 16u;
+        if (z == 0) bits |= 32u;
+    }
+    __shared__ uint32_t s_bits;
+    if (t == 0) s_bits = 0;
+    __syncthreads();
+    if (bits) atomicOr(&s_bits, bits);
+    const int became_varied = __syncthreads_or(wrote) && flag != 0; // every thread has read the flag; s_bits is complete
+#pragma unroll
+    for (int k = 0; k < FILL_WORDS; ++k)
+        if (became_varied || ((differs >> k) & 1u)) row[t + FILL_THREADS * k] = make_uint4(cur[k][0], cur[k][1], cur[k][2], cur[k][3]);
+    if (t == 0) {
+        if (became_varied) flags[s] = 0;
+        *changed = (uint8_t)(s_bits | (became_varied ? 64u : 0u));
+    }
+}
+
+// One CTA per listed slot, the chunk in registers (load_chunk_words).  Every op is applied in registers, skipping words
+// outside its box clipped to the chunk; store_chunk_words writes back what differs.
+__global__ void __launch_bounds__(FILL_THREADS) fill_regions_kernel(uint8_t *voxels, uint8_t *flags, const int32_t *positions,
+                                                                    const RegionOp *__restrict__ ops, int32_t n_ops,
+                                                                    const int32_t *__restrict__ slots, uint8_t *changed) {
+    const int32_t s = slots[blockIdx.x];
+    const uint32_t flag = flags[s];
+    const int t = threadIdx.x, x0 = (t & 1) * 16, y = (t >> 1) & 31, z0 = t >> 6;
+    uint4 *row = reinterpret_cast<uint4 *>(voxels + (size_t)s * VX_CHUNK_VOLUME);
+    uint32_t cur[FILL_WORDS][4], orig[FILL_WORDS][4];
+    load_chunk_words(row, flag, t, cur, orig);
     const int64_t base[3] = {(int64_t)positions[3 * s] * 32, (int64_t)positions[3 * s + 1] * 32, (int64_t)positions[3 * s + 2] * 32};
     int wrote = 0; // some op changed a voxel of this thread's words at its time
     for (int32_t i = 0; i < n_ops; ++i) {
@@ -952,34 +994,98 @@ __global__ void __launch_bounds__(FILL_THREADS) fill_regions_kernel(uint8_t *vox
             }
         }
     }
-    // bits 0..5: a border voxel differs (FaceDir order), 6: some voxel differs
-    uint32_t bits = 0, differs = 0;
+    store_chunk_words(row, flags, s, flag, t, wrote, cur, orig, changed + blockIdx.x);
+}
+
+// vx_world_batch_paste: a validated VxPasteOp; its box is lo .. lo + dims - 1.
+struct PasteOp {
+    int64_t offset;
+    int32_t lo[3], dims[3];
+    uint32_t replace_mask;
+};
+
+// One CTA per listed slot, the chunk in registers as in fill_regions_kernel.  Each op's box is clipped to the chunk; inside
+// it every thread reads the template bytes of its words' x span (one template row segment per word) and applies them.
+__global__ void __launch_bounds__(FILL_THREADS) paste_kernel(uint8_t *voxels, uint8_t *flags, const int32_t *positions,
+                                                             const PasteOp *__restrict__ ops, int32_t n_ops,
+                                                             const uint8_t *__restrict__ templates, const int32_t *__restrict__ slots,
+                                                             uint8_t *changed) {
+    const int32_t s = slots[blockIdx.x];
+    const uint32_t flag = flags[s];
+    const int t = threadIdx.x, x0 = (t & 1) * 16, y = (t >> 1) & 31, z0 = t >> 6;
+    uint4 *row = reinterpret_cast<uint4 *>(voxels + (size_t)s * VX_CHUNK_VOLUME);
+    uint32_t cur[FILL_WORDS][4], orig[FILL_WORDS][4];
+    load_chunk_words(row, flag, t, cur, orig);
+    const int64_t base[3] = {(int64_t)positions[3 * s] * 32, (int64_t)positions[3 * s + 1] * 32, (int64_t)positions[3 * s + 2] * 32};
+    int wrote = 0;
+    for (int32_t i = 0; i < n_ops; ++i) {
+        const PasteOp op = ops[i];
+        int lo[3], hi[3];
+        bool empty = false;
 #pragma unroll
-    for (int k = 0; k < FILL_WORDS; ++k) {
-        const uint32_t d0 = cur[k][0] ^ orig[k][0], d1 = cur[k][1] ^ orig[k][1], d2 = cur[k][2] ^ orig[k][2], d3 = cur[k][3] ^ orig[k][3];
-        if ((d0 | d1 | d2 | d3) == 0) continue;
-        const int z = z0 + 4 * k;
-        differs |= 1u << k;
-        bits |= 64u;
-        if (x0 == 16 && (d3 >> 24) != 0) bits |= 1u;
-        if (x0 == 0 && (d0 & 0xFFu) != 0) bits |= 2u;
-        if (y == 31) bits |= 4u;
-        if (y == 0) bits |= 8u;
-        if (z == 31) bits |= 16u;
-        if (z == 0) bits |= 32u;
-    }
-    __shared__ uint32_t s_bits;
-    if (t == 0) s_bits = 0;
-    __syncthreads();
-    if (bits) atomicOr(&s_bits, bits);
-    const int became_varied = __syncthreads_or(wrote) && flag != 0; // every thread has read the flag; s_bits is complete
+        for (int e = 0; e < 3; ++e) { // the op's box clipped to the chunk, in local coordinates
+            lo[e] = (int)max((int64_t)op.lo[e] - base[e], (int64_t)0);
+            hi[e] = (int)min((int64_t)op.lo[e] + op.dims[e] - 1 - base[e], (int64_t)31);
+            empty |= lo[e] > hi[e];
+        }
+        if (empty || y < lo[1] || y > hi[1] || x0 + 15 < lo[0] || x0 > hi[0]) continue;
+        const int xa = max(lo[0], x0) - x0, xb = min(hi[0], x0 + 15) - x0; // 0..15
+        // template index of (local x0, y, z = 0): t = base + local - lo
+        const int64_t plane = (int64_t)op.dims[1] * op.dims[0];
+        const int64_t at0 = op.offset + (base[2] - op.lo[2]) * plane + (base[1] + y - op.lo[1]) * op.dims[0] + (base[0] + x0 - op.lo[0]);
 #pragma unroll
-    for (int k = 0; k < FILL_WORDS; ++k)
-        if (became_varied || ((differs >> k) & 1u)) row[t + FILL_THREADS * k] = make_uint4(cur[k][0], cur[k][1], cur[k][2], cur[k][3]);
-    if (t == 0) {
-        if (became_varied) flags[s] = 0;
-        changed[blockIdx.x] = (uint8_t)(s_bits | (became_varied ? 64u : 0u));
+        for (int k = 0; k < FILL_WORDS; ++k) {
+            const int z = z0 + 4 * k;
+            if (z < lo[2] || z > hi[2]) continue;
+            const int64_t at = at0 + z * plane;
+#pragma unroll
+            for (int j = 0; j < 16; ++j) {
+                if (j < xa || j > xb) continue;
+                const uint32_t p = __ldg(templates + at + j);
+                const uint32_t sh = 8 * (j & 3), v = (cur[k][j >> 2] >> sh) & 0xFFu;
+                if (p != VX_PASTE_SKIP && ((op.replace_mask >> v) & 1u) && v != p) {
+                    cur[k][j >> 2] = (cur[k][j >> 2] & ~(0xFFu << sh)) | (p << sh);
+                    wrote = 1;
+                }
+            }
+        }
     }
+    store_chunk_words(row, flags, s, flag, t, wrote, cur, orig, changed + blockIdx.x);
+}
+
+// vx_world_batch_copy_region: the box and its chunk table (c0, n: see the header).
+struct CopyBox {
+    int32_t lo[3], dims[3], c0[3], n[3];
+    uint32_t n_table, volume;
+};
+
+// One thread per byte of the packed box, [z][y][x] like the output.  Thread i < n_table also checks table entry i against
+// its slot's position row (n_table <= volume: every chunk of the table holds a voxel of the box on each axis).
+constexpr int COPY_THREADS = 256;
+__global__ void __launch_bounds__(COPY_THREADS) copy_region_kernel(const uint8_t *__restrict__ voxels, const uint8_t *__restrict__ flags,
+                                                                   const int32_t *__restrict__ positions, CopyBox box,
+                                                                   const int32_t *__restrict__ table, uint8_t *__restrict__ out,
+                                                                   uint32_t *stale) {
+    const uint32_t i = blockIdx.x * COPY_THREADS + threadIdx.x;
+    if (i >= box.volume) return;
+    if (i < box.n_table) {
+        const int32_t s = table[i];
+        const uint32_t cx = i % (uint32_t)box.n[0], r = i / (uint32_t)box.n[0];
+        const uint32_t cy = r % (uint32_t)box.n[1], cz = r / (uint32_t)box.n[1];
+        if (s >= 0 && (positions[3 * s] != box.c0[0] + (int32_t)cx || positions[3 * s + 1] != box.c0[1] + (int32_t)cy ||
+                       positions[3 * s + 2] != box.c0[2] + (int32_t)cz))
+            atomicOr(stale, 1u);
+    }
+    const uint32_t x = i % (uint32_t)box.dims[0], r = i / (uint32_t)box.dims[0];
+    const uint32_t y = r % (uint32_t)box.dims[1], z = r / (uint32_t)box.dims[1];
+    const int32_t vx = box.lo[0] + (int32_t)x, vy = box.lo[1] + (int32_t)y, vz = box.lo[2] + (int32_t)z;
+    const int32_t s = table[((vz >> 5) - box.c0[2]) * box.n[1] * box.n[0] + ((vy >> 5) - box.c0[1]) * box.n[0] + ((vx >> 5) - box.c0[0])];
+    uint32_t v = VX_PASTE_SKIP;
+    if (s >= 0) {
+        const uint32_t flag = flags[s];
+        v = flag ? flag - 1 : voxels[(size_t)s * VX_CHUNK_VOLUME + (vz & 31) * 1024 + (vy & 31) * 32 + (vx & 31)];
+    }
+    out[i] = (uint8_t)v;
 }
 
 } // namespace
@@ -1562,6 +1668,103 @@ int vx_world_batch_read_voxels(VxContext *ctx, const VxMeshBatch *b, const int32
                                          cudaMemcpyDeviceToHost, ctx->stream));
         VX_CUDA(ctx, cudaMemcpyAsync(flags_out + i, b->world_flags.as<uint8_t>() + s, 1, cudaMemcpyDeviceToHost, ctx->stream));
     }
+    VX_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+    return VX_OK;
+}
+
+int vx_world_batch_copy_region(VxContext *ctx, const VxMeshBatch *b, const int32_t lo[3], const int32_t dims[3], const int32_t *chunk_slots,
+                               uint8_t *out) {
+    int rc = world_check_slots(ctx, b, nullptr, 0, "vx_world_batch_copy_region: bad argument");
+    if (rc != VX_OK) return rc;
+    if (!lo || !dims || !chunk_slots || !out) return vx_fail(ctx, VX_ERR_INVALID, "vx_world_batch_copy_region: bad argument");
+    constexpr int32_t COORD = 1 << 29, MAX_DIM = 1024;
+    CopyBox box;
+    for (int e = 0; e < 3; ++e) {
+        if (dims[e] < 1 || dims[e] > MAX_DIM) return vx_fail(ctx, VX_ERR_INVALID, "vx_world_batch_copy_region: dims out of range");
+        if (lo[e] < -COORD || lo[e] > COORD - (dims[e] - 1)) return vx_fail(ctx, VX_ERR_INVALID, "vx_world_batch_copy_region: coordinate out of range");
+        box.lo[e] = lo[e];
+        box.dims[e] = dims[e];
+        box.c0[e] = lo[e] >> 5;
+        box.n[e] = ((lo[e] + dims[e] - 1) >> 5) - box.c0[e] + 1;
+    }
+    box.n_table = (uint32_t)box.n[0] * (uint32_t)box.n[1] * (uint32_t)box.n[2];
+    box.volume = (uint32_t)dims[0] * (uint32_t)dims[1] * (uint32_t)dims[2];
+    for (uint32_t i = 0; i < box.n_table; ++i)
+        if (chunk_slots[i] < -1 || chunk_slots[i] >= b->n_chunks) return vx_fail(ctx, VX_ERR_INVALID, "vx_world_batch_copy_region: slot out of range");
+    VX_CUDA(ctx, cudaSetDevice(ctx->device));
+    // staged: the chunk table, the stale-table word, then the packed box the kernel writes
+    const size_t table_bytes = sizeof(int32_t) * box.n_table;
+    VX_CUDA(ctx, ctx->tmp_a.reserve(table_bytes + sizeof(uint32_t) + box.volume));
+    uint8_t *d = ctx->tmp_a.as<uint8_t>();
+    uint32_t *d_stale = reinterpret_cast<uint32_t *>(d + table_bytes);
+    VX_CUDA(ctx, cudaMemcpyAsync(d, chunk_slots, table_bytes, cudaMemcpyHostToDevice, ctx->stream));
+    VX_CUDA(ctx, cudaMemsetAsync(d_stale, 0, sizeof(uint32_t), ctx->stream));
+    copy_region_kernel<<<(box.volume + COPY_THREADS - 1) / COPY_THREADS, COPY_THREADS, 0, ctx->stream>>>(
+        b->world_voxels.as<uint8_t>(), b->world_flags.as<uint8_t>(), b->positions.as<int32_t>(), box, reinterpret_cast<const int32_t *>(d),
+        d + table_bytes + sizeof(uint32_t), d_stale);
+    VX_CHECK_LAUNCH(ctx);
+    uint32_t stale = 0;
+    VX_CUDA(ctx, cudaMemcpyAsync(&stale, d_stale, sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->stream));
+    VX_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+    if (stale) return vx_fail(ctx, VX_ERR_INVALID, "vx_world_batch_copy_region: a slot's position is not the chunk it is listed for");
+    VX_CUDA(ctx, cudaMemcpyAsync(out, d + table_bytes + sizeof(uint32_t), box.volume, cudaMemcpyDeviceToHost, ctx->stream));
+    VX_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+    return VX_OK;
+}
+
+int vx_world_batch_paste(VxContext *ctx, VxMeshBatch *b, const VxPasteOp *ops, int32_t n_ops, const uint8_t *templates, int64_t n_template_bytes,
+                         const int32_t *slots, int32_t n_slots, uint8_t *changed_out) {
+    int rc = world_check_slots(ctx, b, slots, n_slots, "vx_world_batch_paste: bad argument");
+    if (rc != VX_OK) return rc;
+    if (n_ops < 0 || (n_ops > 0 && !ops) || n_template_bytes < 0 || (n_template_bytes > 0 && !templates) || (n_slots > 0 && !changed_out))
+        return vx_fail(ctx, VX_ERR_INVALID, "vx_world_batch_paste: bad argument");
+    std::vector<uint8_t> listed((size_t)b->n_chunks, 0);
+    for (int32_t i = 0; i < n_slots; ++i)
+        if (listed[slots[i]]++) return vx_fail(ctx, VX_ERR_INVALID, "vx_world_batch_paste: slot listed twice");
+    constexpr int32_t COORD = 1 << 29, MAX_DIM = 1024;
+    std::vector<PasteOp> dev((size_t)n_ops);
+    for (int32_t i = 0; i < n_ops; ++i) {
+        const VxPasteOp &o = ops[i];
+        if (o.replace_mask > 15) return vx_fail(ctx, VX_ERR_INVALID, "vx_world_batch_paste: replace mask out of range");
+        int64_t volume = 1;
+        for (int e = 0; e < 3; ++e) {
+            if (o.dims[e] < 1 || o.dims[e] > MAX_DIM) return vx_fail(ctx, VX_ERR_INVALID, "vx_world_batch_paste: dims out of range");
+            if (o.origin[e] < -COORD || o.origin[e] > COORD - (o.dims[e] - 1))
+                return vx_fail(ctx, VX_ERR_INVALID, "vx_world_batch_paste: coordinate out of range");
+            volume *= o.dims[e];
+        }
+        if (o.offset < 0 || o.offset > n_template_bytes - volume) return vx_fail(ctx, VX_ERR_INVALID, "vx_world_batch_paste: template out of range");
+        const uint8_t *p = templates + o.offset;
+        int bad = 0;
+        for (int64_t j = 0; j < volume; ++j) bad |= p[j] > 3 && p[j] != VX_PASTE_SKIP;
+        if (bad) return vx_fail(ctx, VX_ERR_INVALID, "vx_world_batch_paste: template byte other than 0..3 or VX_PASTE_SKIP");
+        PasteOp &d = dev[(size_t)i];
+        d.offset = o.offset;
+        for (int e = 0; e < 3; ++e) {
+            d.lo[e] = o.origin[e];
+            d.dims[e] = o.dims[e];
+        }
+        d.replace_mask = o.replace_mask;
+    }
+    if (n_slots == 0) return VX_OK;
+    if (n_ops == 0) {
+        memset(changed_out, 0, (size_t)n_slots);
+        return VX_OK;
+    }
+    VX_CUDA(ctx, cudaSetDevice(ctx->device));
+    // staged: ops, slots, the change bytes the kernel writes, then the templates
+    const size_t ops_bytes = sizeof(PasteOp) * dev.size(), slot_bytes = sizeof(int32_t) * (size_t)n_slots;
+    const size_t tmpl_at = (ops_bytes + slot_bytes + (size_t)n_slots + 15) & ~(size_t)15;
+    VX_CUDA(ctx, ctx->tmp_a.reserve(tmpl_at + (size_t)n_template_bytes));
+    uint8_t *d = ctx->tmp_a.as<uint8_t>();
+    VX_CUDA(ctx, cudaMemcpyAsync(d, dev.data(), ops_bytes, cudaMemcpyHostToDevice, ctx->stream));
+    VX_CUDA(ctx, cudaMemcpyAsync(d + ops_bytes, slots, slot_bytes, cudaMemcpyHostToDevice, ctx->stream));
+    VX_CUDA(ctx, cudaMemcpyAsync(d + tmpl_at, templates, (size_t)n_template_bytes, cudaMemcpyHostToDevice, ctx->stream));
+    paste_kernel<<<(unsigned)n_slots, FILL_THREADS, 0, ctx->stream>>>(
+        b->world_voxels.as<uint8_t>(), b->world_flags.as<uint8_t>(), b->positions.as<int32_t>(), reinterpret_cast<const PasteOp *>(d), n_ops,
+        d + tmpl_at, reinterpret_cast<const int32_t *>(d + ops_bytes), d + ops_bytes + slot_bytes);
+    VX_CHECK_LAUNCH(ctx);
+    VX_CUDA(ctx, cudaMemcpyAsync(changed_out, d + ops_bytes + slot_bytes, (size_t)n_slots, cudaMemcpyDeviceToHost, ctx->stream));
     VX_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
     return VX_OK;
 }

@@ -21,6 +21,7 @@ Pos = Tuple[int, int, int]
 CHUNK_SIZE = 32
 FACE_OFFSETS = ((1, 0, 0), (-1, 0, 0), (0, 1, 0), (0, -1, 0), (0, 0, 1), (0, 0, -1))  # FaceDir order, mesh.rs:136-143
 NBR_NONE = -1
+PASTE_SKIP = _lib.PASTE_SKIP
 
 
 class WorldConfig:
@@ -76,6 +77,24 @@ def region_contains(op: np.ndarray, voxels: np.ndarray) -> np.ndarray:
     return near & ((np.where(near[:, None], d, 0) ** 2).sum(axis=1) <= int(op["radius_sq"]))
 
 
+PASTE_MAX_DIM = 1024  # the largest extent per axis of vx_world_batch_copy_region / vx_world_batch_paste
+
+
+def _paste_box(lo, dims) -> Tuple[np.ndarray, np.ndarray]:
+    """lo and dims as int64 (3,); ValueError for a box vx_world_batch_copy_region / _paste would refuse."""
+    lo, dims = np.asarray(lo, dtype=np.int64).reshape(3), np.asarray(dims, dtype=np.int64).reshape(3)
+    if (dims < 1).any() or (dims > PASTE_MAX_DIM).any():
+        raise ValueError(f"copy / paste boxes are 1..{PASTE_MAX_DIM} voxels per axis")
+    if (np.abs(lo) > REGION_COORD).any() or (np.abs(lo + dims - 1) > REGION_COORD).any():
+        raise ValueError("copy / paste coordinates are limited to [-2^29, 2^29]")
+    return lo, dims
+
+
+def _chunk_starts(lo: int, n: int) -> np.ndarray:
+    """Indices 0 <= i < n along one axis of a box starting at world voxel lo where a new chunk begins (0 included)."""
+    return np.unique(np.concatenate([[0], np.arange((-lo) % CHUNK_SIZE, n, CHUNK_SIZE)])).astype(np.intp)
+
+
 class _DeviceWorld:
     """The vx_world_batch_* calls (block and region edits included), vx_world_raycast and vx_world_move_boxes; tests
     substitute a recorder for it to check the host logic without a GPU."""
@@ -128,6 +147,22 @@ class _DeviceWorld:
                                                                api._p(voxels), api._p(flags)))
         return voxels, flags
 
+    def copy_region(self, lo: np.ndarray, dims: np.ndarray, chunk_slots: np.ndarray) -> np.ndarray:
+        """The box lo .. lo + dims - 1 as (dims[2], dims[1], dims[0]) uint8; chunk_slots [cz][cy][cx] (-1 = not loaded)."""
+        lo, dims = np.ascontiguousarray(lo, dtype=np.int32), np.ascontiguousarray(dims, dtype=np.int32)
+        out = np.empty(tuple(int(d) for d in dims[::-1]), dtype=np.uint8)
+        table = np.ascontiguousarray(chunk_slots, dtype=np.int32)
+        self.ctx.check(self.ctx.lib.vx_world_batch_copy_region(self.ctx.handle, self.batch.handle, api._p(lo), api._p(dims), api._p(table),
+                                                               api._p(out)))
+        return out
+
+    def paste(self, ops: np.ndarray, templates: np.ndarray, slots: np.ndarray) -> np.ndarray:
+        """ops: api.PASTE_OP_DTYPE records into the uint8 buffer templates; returns the change bits per slot."""
+        changed = np.zeros(slots.size, dtype=np.uint8)
+        self.ctx.check(self.ctx.lib.vx_world_batch_paste(self.ctx.handle, self.batch.handle, api._p(ops), int(ops.size), api._p(templates),
+                                                         C.c_int64(templates.size), api._p(slots), int(slots.size), api._p(changed)))
+        return changed
+
     def raycast(self, origins: np.ndarray, dirs: np.ndarray, start_slots: np.ndarray, max_t: float) -> np.ndarray:
         hits = np.zeros(start_slots.size, dtype=api.RAY_HIT_DTYPE)
         self.ctx.check(self.ctx.lib.vx_world_raycast(self.ctx.handle, self.batch.handle, api._p(origins), api._p(dirs), api._p(start_slots),
@@ -160,6 +195,12 @@ class World:
         # of the fills that changed it: replayed, before `edits`, when the chunk is generated anew
         self.fills: List[np.ndarray] = []
         self._fills_at: Dict[Pos, List[int]] = {}
+        # pastes (paste; an api.PASTE_OP_DTYPE record with offset 0 and its own copy of the template) in issue order, how many
+        # fills were issued before each, and per chunk position the indices of the pastes that changed it: replayed with the
+        # fills, in issue order, before `edits`
+        self.pastes: List[Tuple[np.ndarray, np.ndarray]] = []
+        self._pastes_after: List[int] = []
+        self._pastes_at: Dict[Pos, List[int]] = {}
         self._free: List[int] = list(range(self.capacity - 1, -1, -1))
         self.last_camera_chunk: Optional[Pos] = None
         self.generated_last_update: List[Pos] = []
@@ -248,13 +289,9 @@ class World:
         flags = self.device.generate(slots, np.array(new, dtype=np.int32).reshape(-1, 3))
         for p, f in zip(new, flags.tolist()):
             self.uniform_flags[p] = int(f)
-        refill = [p for p in new if p in self._fills_at]
-        if refill:
-            ops = np.stack([self.fills[i] for i in sorted({i for p in refill for i in self._fills_at[p]})])
-            changed = self.device.fill_regions(ops, np.array([self.chunks[p] for p in refill], dtype=np.int32))
-            for p, c in zip(refill, changed.tolist()):
-                if c & _lib.REGION_CHANGED:
-                    self.uniform_flags[p] = 0
+        replay = [p for p in new if p in self._fills_at or p in self._pastes_at]
+        if replay:
+            self._replay(replay)
         edited = [p for p in new if p in self.edits]
         if edited:
             self._apply_edits([(p, i, t) for p in edited for i, t in self.edits[p].items()])
@@ -262,6 +299,35 @@ class World:
         for p in new:  # the chunks next to a new one now have a neighbour there
             touched += [(p[0] + o[0], p[1] + o[1], p[2] + o[2]) for o in FACE_OFFSETS]
         self._push_neighbor_rows(touched)
+
+    def _replay(self, positions: List[Pos]):
+        """Replay the fills and pastes that changed `positions` (just generated) in issue order: each run of consecutive
+        fills in one fill_regions call, each run of consecutive pastes in one paste call, over the positions that one of
+        the run's ops changed.  Exact (DESIGN §3.3): both are per-voxel functions of the voxel's old type."""
+        fills = sorted({i for p in positions for i in self._fills_at.get(p, ())})
+        pastes = sorted({j for p in positions for j in self._pastes_at.get(p, ())})
+        # paste j was issued after fills 0 .. _pastes_after[j] - 1, so it sorts between fill _pastes_after[j] - 1 and the next
+        order = sorted([(i, 1, i) for i in fills] + [(self._pastes_after[j], 0, j) for j in pastes])
+        runs: List[Tuple[int, List[int]]] = []
+        for _, is_fill, i in order:
+            if runs and runs[-1][0] == is_fill:
+                runs[-1][1].append(i)
+            else:
+                runs.append((is_fill, [i]))
+        for is_fill, run in runs:
+            at, members = (self._fills_at, set(run)) if is_fill else (self._pastes_at, set(run))
+            ps = [p for p in positions if members.intersection(at.get(p, ()))]
+            slots = np.array([self.chunks[p] for p in ps], dtype=np.int32)
+            if is_fill:
+                changed = self.device.fill_regions(np.stack([self.fills[i] for i in run]), slots)
+            else:
+                ops = np.stack([self.pastes[j][0] for j in run])
+                sizes = [self.pastes[j][1].size for j in run]
+                ops["offset"] = np.concatenate([[0], np.cumsum(sizes)[:-1]])
+                changed = self.device.paste(ops, np.concatenate([self.pastes[j][1].reshape(-1) for j in run]), slots)
+            for p, c in zip(ps, changed.tolist()):
+                if c & _lib.REGION_CHANGED:
+                    self.uniform_flags[p] = 0
 
     def _grow(self, capacity: int):
         if capacity <= self.capacity:
@@ -397,6 +463,79 @@ class World:
                 hit = region_contains(op, v) & (((int(op["replace_mask"]) >> types) & 1) == 1)
                 for i in idx[hit].tolist():
                     e[i] = int(op["block_type"])
+        return sorted(dirty)
+
+    # ---- copy and paste (vx_world_batch_copy_region, vx_world_batch_paste) ------------------------------------------
+    def copy_region(self, lo, hi) -> np.ndarray:
+        """The voxels of the box lo..hi (world voxel coordinates, both corners inclusive, 1..1024 voxels per axis) as uint8
+        indexed [z, y, x], PASTE_SKIP where the chunk is not loaded: one device call (vx_world_batch_copy_region).  Unloaded
+        space is never an error, so the result can be pasted back as it is."""
+        lo = np.asarray(lo, dtype=np.int64).reshape(3)
+        lo, dims = _paste_box(lo, np.asarray(hi, dtype=np.int64).reshape(3) - lo + 1)
+        c0, c1 = lo >> 5, (lo + dims - 1) >> 5
+        table = np.array([[[self.chunks.get((x, y, z), -1) for x in range(c0[0], c1[0] + 1)] for y in range(c0[1], c1[1] + 1)]
+                          for z in range(c0[2], c1[2] + 1)], dtype=np.int32)
+        return self.device.copy_region(lo, dims, table)
+
+    def paste(self, template, origin, replace: Optional[Iterable[int]] = None) -> List[Pos]:
+        """Stamp template ((sz, sy, sx) uint8, indexed [z, y, x]) with byte (0, 0, 0) on world voxel origin: a byte 0..3 sets
+        its voxel to that type if the voxel's type is in `replace` (block types; None = all four); PASTE_SKIP leaves it
+        alone.  Transparent air is np.where(t == 0, PASTE_SKIP, t); rotations are np.rot90(t, k, axes=(0, 2)).  Exact
+        semantics in include/vx_b200.h (vx_world_batch_paste).  Every chunk where the template has a byte other than
+        PASTE_SKIP must be loaded (KeyError otherwise, before anything changes); the others are not touched, so a copy
+        taken across unloaded space can be pasted back.  The paste is recorded with its own copy of the template and comes
+        back when a chunk is unloaded and generated again (with the fills, in issue order, then `edits`, into which every
+        paste is folded).  Nothing is re-meshed: returns the positions whose meshes may change, as fill_ball does."""
+        t = np.asarray(template)
+        if t.ndim != 3 or not np.issubdtype(t.dtype, np.integer):
+            raise ValueError("a template is a (sz, sy, sx) array of block types")
+        origin, dims = _paste_box(origin, t.shape[::-1])
+        if ((t > 3) & (t != PASTE_SKIP)).any() or (t < 0).any():
+            raise ValueError("template bytes are block types 0..3 or PASTE_SKIP")
+        types = range(4) if replace is None else [int(v) for v in replace]
+        if any(not 0 <= v <= 3 for v in types):
+            raise ValueError("block types are 0..3")
+        t = np.array(t, dtype=np.uint8, order="C")  # the record's own copy
+        # the chunks under at least one byte other than PASTE_SKIP
+        starts = [_chunk_starts(int(origin[e]), int(dims[e])) for e in range(3)]
+        solid = (t != PASTE_SKIP).view(np.uint8)
+        for axis, e in ((0, 2), (1, 1), (2, 0)):
+            solid = np.maximum.reduceat(solid, starts[e], axis=axis)
+        c0 = origin >> 5
+        touched = [(int(c0[0] + i), int(c0[1] + j), int(c0[2] + k)) for k, j, i in zip(*np.nonzero(solid))]
+        missing = sorted(p for p in touched if p not in self.chunks)
+        if missing:
+            raise KeyError(f"paste: chunks not loaded: {missing[:16]}{' ...' if len(missing) > 16 else ''}")
+        if not touched:
+            return []
+        op = np.zeros((), dtype=api.PASTE_OP_DTYPE)
+        op["origin"], op["dims"], op["replace_mask"] = origin, dims, sum(1 << v for v in set(types))
+        changed = self.device.paste(op.reshape(1), t.reshape(-1), np.array([self.chunks[p] for p in touched], dtype=np.int32))
+        k = len(self.pastes)
+        self.pastes.append((op, t))
+        self._pastes_after.append(len(self.fills))
+        dirty = set()
+        for p, c in zip(touched, changed.tolist()):
+            if not c & _lib.REGION_CHANGED:
+                continue  # unchanged: replaying the paste there would change nothing but voxels that `edits` sets anyway
+            self._pastes_at.setdefault(p, []).append(k)
+            self.uniform_flags[p] = 0
+            dirty.add(p)
+            for f, o in enumerate(FACE_OFFSETS):
+                q = (p[0] + o[0], p[1] + o[1], p[2] + o[2])
+                if (c >> f) & 1 and q in self.chunks:
+                    dirty.add(q)
+            e = self.edits.get(p)
+            if e:  # fold: an edited voxel under a byte other than PASTE_SKIP whose type is in the mask now holds that byte
+                idx = np.fromiter(e.keys(), dtype=np.int64, count=len(e))
+                types_now = np.fromiter(e.values(), dtype=np.int64, count=len(e))
+                tv = np.stack([idx & 31, (idx >> 5) & 31, idx >> 10], axis=1) + np.array(p, dtype=np.int64) * CHUNK_SIZE - origin
+                inside = ((tv >= 0) & (tv < dims)).all(axis=1)
+                tv = np.where(inside[:, None], tv, 0)
+                b = t[tv[:, 2], tv[:, 1], tv[:, 0]].astype(np.int64)
+                hit = inside & (b != PASTE_SKIP) & (((int(op["replace_mask"]) >> types_now) & 1) == 1)
+                for i, v in zip(idx[hit].tolist(), b[hit].tolist()):
+                    e[i] = v
         return sorted(dirty)
 
     def chunk_voxels(self, pos) -> Tuple[int, np.ndarray]:

@@ -286,6 +286,51 @@ VX_API int vx_world_batch_fill_regions(VxContext *ctx, VxMeshBatch *b, const VxR
 VX_API int vx_world_batch_read_voxels(VxContext *ctx, const VxMeshBatch *b, const int32_t *slots, int32_t n, uint8_t *voxels_out,
                                       uint8_t *flags_out);
 
+/* ---- copy and paste: read a box of voxels back, stamp block patterns into a world batch -----------------------------
+ * The exact semantics, which the CPU oracle (tests/paste_oracle.c: vxo_copy_region, vxo_paste) restates statement for
+ * statement, all in integer arithmetic.  ">> 5" is an arithmetic shift (floor division by 32); a world voxel v lies in
+ * chunk v >> 5 at local v & 31, index z*1024 + y*32 + x.
+ *
+ * vx_world_batch_copy_region: out (host, dims[2] * dims[1] * dims[0] bytes) receives the box lo .. lo + dims - 1:
+ *   - c0 = lo >> 5, c1 = (lo + dims - 1) >> 5, n = c1 - c0 + 1 per axis; chunk_slots holds n[2] * n[1] * n[0] entries, the
+ *     slot of chunk c0 + (i, j, k) at [(k * n[1] + j) * n[0] + i], or -1 for a chunk that is not loaded.
+ *   - out[(z * dims[1] + y) * dims[0] + x], for voxel v = lo + (x, y, z) with entry s = the entry of chunk v >> 5:
+ *     VX_PASTE_SKIP if s = -1; else flag - 1 if the slot's Uniform flag is not 0 (its rows are not read); else the byte at
+ *     index (v & 31) of the slot's row.
+ *   - VX_ERR_INVALID, before anything is written, for: a batch that is not a world batch; a dims[e] outside [1, 1024]; a
+ *     coordinate of lo or of lo + dims - 1 outside [-2^29, 2^29]; an entry outside [-1, capacity); an entry s >= 0 whose
+ *     position row (vx_world_batch_generate / _assign) is not the chunk it is listed for -- a stale table.
+ *   One gather kernel writes the packed box on the device, then one copy brings exactly the box back.  Synchronous.
+ *
+ * vx_world_batch_paste: each listed slot applies ops 0 .. n_ops-1 in order to its own voxels (a later op wins where two
+ * overlap).  Op i's template is the dims[2] x dims[1] x dims[0] bytes at templates + offset, indexed [z][y][x]:
+ *   - voxel (x, y, z) of a slot is world voxel v = position * 32 + local; with t = v - origin, the op covers v iff
+ *     0 <= t[e] < dims[e] on every axis, and its byte is p = templates[offset + (t[2] * dims[1] + t[1]) * dims[0] + t[0]].
+ *   - p = VX_PASTE_SKIP leaves the voxel as it is; p in 0..3 sets it to p if its current type t has bit t set in
+ *     replace_mask; voxels no op covers are never written.
+ *   - VX_ERR_INVALID, before anything changes, for: a batch that is not a world batch; a slot outside [0, capacity) or
+ *     listed twice; replace_mask > 15; a dims[e] outside [1, 1024]; a coordinate of origin or of origin + dims - 1 outside
+ *     [-2^29, 2^29]; offset < 0 or offset + dims[0] * dims[1] * dims[2] > n_template_bytes; a byte of an op's template
+ *     outside {0, 1, 2, 3, VX_PASTE_SKIP} (checked on the host: bytes no op covers are not looked at).
+ *   - Uniform slots and changed_out[i] exactly as in vx_world_batch_fill_regions: a Uniform slot turns Varied at the first
+ *     op that changes one of its voxels (covered, p != SKIP, its type in the mask, and p differs from it), and stays
+ *     Varied; one no op changes keeps its flag and its rows are not written.  Bit 6: the voxels or the flag differ from
+ *     before the call; bit f (0..5, FaceDir order): a voxel on that border plane differs.
+ * Nothing is re-meshed (see vx_world_batch_fill_regions for what to re-mesh).  The templates are copied to the device
+ * whole (n_template_bytes).  Stream ordered; synchronises before it returns. */
+enum { VX_PASTE_SKIP = 0xFF };
+typedef struct {
+    int64_t offset;        /* byte offset of this op's template in `templates` */
+    int32_t origin[3];     /* world voxel that template byte (0, 0, 0) lands on */
+    int32_t dims[3];       /* template extent in x, y, z: 1..1024 each */
+    uint8_t replace_mask;  /* bit t set: voxels of type t may be overwritten (0xF = all) */
+    uint8_t pad[7];
+} VxPasteOp; /* 40 bytes */
+VX_API int vx_world_batch_copy_region(VxContext *ctx, const VxMeshBatch *b, const int32_t lo[3], const int32_t dims[3],
+                                      const int32_t *chunk_slots, uint8_t *out);
+VX_API int vx_world_batch_paste(VxContext *ctx, VxMeshBatch *b, const VxPasteOp *ops, int32_t n_ops, const uint8_t *templates,
+                                int64_t n_template_bytes, const int32_t *slots, int32_t n_slots, uint8_t *changed_out);
+
 /* ---- ray casting through a world batch (picking) -------------------------------------------------------------------
  * One ray per thread, an Amanatides-Woo walk over the voxels the world batch holds; the exact semantics, which the CPU
  * oracle (tests/ray_oracle.c: vxo_raycast) restates statement for statement, so that both give identical bits:
